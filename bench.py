@@ -7,7 +7,7 @@ synthetic 2D LiDAR pairs, 65,536 pairs x 360 points, 30 forced iterations
 by oracle.icp_oracle.synth_room_batch (seed = 1234 + pair index).  Weak scaling: every
 rank aligns its own 65,536 pairs (pair indices rank*65536 ...), no data-path collective.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference      # CPU arm: the oracle port on all host cores
 
@@ -67,7 +67,35 @@ def parse():
                     help="scan2map: replay the 30-iteration loop as one CUDA graph (default with the peer exchange)")
     ap.add_argument("--no-s2m-graph", dest="s2m_graph", action="store_false",
                     help="scan2map: launch the 60 kernels of an alignment from the host loop")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="pairs workload: write what the last timed step computed on rank 0 (the AlignResult "
+                         "fields) to DIR/<field>.npy as float64, so that two builds can be compared on the same "
+                         "seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "pairs"):
+        ap.error("--dump-outputs covers the headline workload only (--impl b200 --workload pairs)")
+    return args
+
+
+DUMP_BYTES = 60 << 20          # keeps the files, .npy headers included, under 64 MB (10^6 B)
+
+
+def dump_outputs(directory, res):
+    """Every [P, ...] field of ``res`` as float64 (int32 counts are exact in float64); above DUMP_BYTES
+    in all, a fixed seeded sample of the pairs, whose indices go to pair_index.npy."""
+    fields = {f: getattr(res, f).cpu().numpy().astype(np.float64)
+              for f in ("pose_total", "pose_last", "error", "rmse", "inliers", "iterations")}
+    n = len(fields["pose_total"])
+    row_bytes = sum(a[0].nbytes for a in fields.values())
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+        fields = {f: a[rows] for f, a in fields.items()}
+        fields["pair_index"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in fields.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -348,6 +376,8 @@ def run_b200(args):
     total_ms = max_over_ranks(t_all0.elapsed_time(t_all1))
     kernel_ms = float(np.mean([e0.elapsed_time(e1) for e0, e1 in evs]))     # per-launch duration
     assert bool(torch.all(out.iterations == ITERS)), "forced-iteration run did not run 30 iterations"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     # untimed diagnostic launch: how many pair evaluations did the (exactly pruned) sweep execute?
     stats = m.align_pairs(src, tgt, max_iterations=ITERS, tolerance=-1.0, want_stats=True)
     torch.cuda.synchronize()

@@ -95,24 +95,6 @@ def test_filter_points_bit_exact(gold):
         assert 0 < len(kept) < len(gold[f"filter_{i}_pts"])
 
 
-def test_against_live_reference_when_present():
-    """In the build container the unmodified process.py is importable: compare on fresh inputs."""
-    from oracle import ref_loader
-    if not os.path.isfile(os.path.join(ref_loader.REFERENCE_ROOT, "duc", "ICP_LIDAR", "process.py")):
-        pytest.skip("reference tree not present (GPU box)")
-    ref = ref_loader.load_reference_process()
-    pts, rob = occ.synth_replay(7, 6, beams=90)
-    o_r = np.full((300, 320), 0.5, dtype=np.float32)
-    i_r = np.full((300, 320, 3), 128, dtype=np.uint8)
-    o_o, i_o = o_r.copy(), i_r.copy()
-    ref.update_occupancy_map.occupancy_probs = o_r
-    for f in range(len(pts)):
-        ref.update_occupancy_map(i_r, pts[f], rob[f], (160, 150), 30)
-        occ.update_occupancy_map_c(o_o, i_o, pts[f], rob[f], (160, 150), 30)
-    del ref.update_occupancy_map.occupancy_probs
-    assert np.array_equal(o_r.view(np.uint32), o_o.view(np.uint32)) and np.array_equal(i_r, i_o)
-
-
 def test_slam_oracle_composition_tracks_the_recording(packed):
     """oracle/slam_oracle.py (the order of slam_offline.py:318-455 over the pinned oracles): the
     first 80 scans are all registered, the map grows and is re-sampled, free space is carved."""

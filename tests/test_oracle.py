@@ -4,10 +4,8 @@ import os
 import zlib
 
 import numpy as np
-import pytest
 
 from oracle import icp_oracle as orc
-from oracle import ref_loader
 
 
 def test_circle_demo_matches_reference_bitwise(golden):
@@ -126,21 +124,19 @@ def test_synthetic_generator_is_seeded_and_recoverable():
     assert np.linalg.norm(r.t_tot - tr) < 30.0
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
-def test_live_reference_equals_oracle(cart_scans):
-    """Build container only: run the unmodified reference side by side."""
-    ref = ref_loader.load_reference_icp()
+def test_reference_form_and_best_fit_match_recorded_reference(golden, cart_scans):
+    """icp_reference_form returns what the unmodified icp() returned, and best_fit_transform
+    reproduces the reference's best_fit_transform(A, src) (tests/golden/make_golden.py) bit for
+    bit, on the reference's own full src arrays of the spot pairs."""
     for p in (2, 99, 672, 1062, 1500):
         A, B = cart_scans[p + 1], cart_scans[p]
-        src, R, t = ref.icp(A, B, 30, 1e-5)
-        o = orc.icp_extended(A, B, 30, 1e-5)
-        assert np.array_equal(src, o.src) and np.array_equal(R, o.R_last) and np.array_equal(t, o.t_last)
-        s2, R2, t2 = orc.icp_reference_form(A, B, 30, 1e-5)
-        assert np.array_equal(src, s2)
-    P, Q = cart_scans[5][:100], cart_scans[6][:100]
-    Rr, tr = ref.best_fit_transform(P, Q)
-    Ro, to = orc.best_fit_transform(P, Q)
-    assert np.array_equal(Rr, Ro) and np.array_equal(tr, to)
+        src, R, t = orc.icp_reference_form(A, B, 30, 1e-5)
+        assert zlib.crc32(np.ascontiguousarray(src).tobytes()) == golden["pair_src_crc32"][p], f"pair {p}"
+        assert np.array_equal(R, golden["pair_R_last"][p]) and np.array_equal(t, golden["pair_t_last"][p])
+    for k in golden["spot_pairs"]:
+        Rc, tc = orc.best_fit_transform(cart_scans[k], golden[f"spot_src_{k}"])
+        assert np.arctan2(Rc[1, 0], Rc[0, 0]) == golden["pair_theta_tot"][k - 1], f"pair {k}"
+        assert np.array_equal(tc, golden["pair_t_tot"][k - 1]), f"pair {k}"
 
 
 def test_c_oracle_matches_numpy_oracle(cart_scans):
