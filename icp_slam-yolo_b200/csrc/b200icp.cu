@@ -1598,7 +1598,7 @@ __global__ void __launch_bounds__(32, B200ICP_PAIR_RESIDENT_WARPS) nn_warp_kerne
 
 // ------------------------------------------------------------------------------------
 // kernel: best_fit_transform(A, B) for matched rows (icp.py:5-26), one warp per pair:
-// centroids, centred 2x2 cross-covariance (single pass relative to B's first point),
+// centroids, centred 2x2 cross-covariance (single pass, each cloud relative to its first point),
 // closed-form proper rotation, t = cB - R cA.
 // ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(32) best_fit_warp_kernel(const KernelArgs a) {
@@ -1615,12 +1615,15 @@ __global__ void __launch_bounds__(32) best_fit_warp_kernel(const KernelArgs a) {
     if (lane == 0) { pose[0] = 1; pose[1] = 0; pose[2] = 0; pose[3] = 1; pose[4] = 0; pose[5] = 0; }
     return;
   }
+  // each cloud relative to its own first point: the single-pass sums then cancel only as much as
+  // the spread of the cloud, however far apart the two clouds are
+  const double2 oa = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch);
   const double2 o = load_point(pr.tgt_points, pr.dtype, trow * pr.tgt_pitch);
   double r[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   for (int i = lane; i < n; i += 32) {
     const double2 s = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i);
     const double2 b = load_point(pr.tgt_points, pr.dtype, trow * pr.tgt_pitch + i);
-    const double ax = s.x - o.x, ay = s.y - o.y, qx = b.x - o.x, qy = b.y - o.y;
+    const double ax = s.x - oa.x, ay = s.y - oa.y, qx = b.x - o.x, qy = b.y - o.y;
     r[0] += ax; r[1] += ay; r[2] += qx; r[3] += qy;
     r[4] = fma(ax, qx, r[4]); r[5] = fma(ax, qy, r[5]);
     r[6] = fma(ay, qx, r[6]); r[7] = fma(ay, qy, r[7]);
@@ -1639,7 +1642,7 @@ __global__ void __launch_bounds__(32) best_fit_warp_kernel(const KernelArgs a) {
     const double h2 = fma(num, num, den * den);
     double cs = 1.0, sn = 0.0;
     if (h2 > 0.0) { const double rh = rsqrt(h2); cs = den * rh; sn = num * rh; }
-    const double cax = o.x + max_, cay = o.y + may_;
+    const double cax = oa.x + max_, cay = oa.y + may_;
     pose[0] = cs; pose[1] = -sn; pose[2] = sn; pose[3] = cs;
     pose[4] = (o.x + mbx) - (cs * cax - sn * cay);          // icp.py:25
     pose[5] = (o.y + mby) - (sn * cax + cs * cay);
@@ -1707,9 +1710,9 @@ constexpr int kSelBlock = 1024;      // points per CTA (256 threads x 4)
 __device__ __forceinline__ bool select_keep(const void* points, int dtype, int64_t i, int mode,
                                             const double* key, double cx, double cy, double thr) {
   if (mode == 0) return key[i] < thr;
-  const double2 q = load_point(points, dtype, i);
-  const double dx = q.x - cx, dy = q.y - cy;
-  return dx * dx + dy * dy < thr;                       // mainn.py:302  distances_sq < R^2
+  // mainn.py:302  distances_sq < R^2, rounded as NumPy rounds it (a contracted FMA decides points
+  // within an ulp of the circle differently)
+  return dist2_f64(cx, cy, load_point(points, dtype, i)) < thr;
 }
 
 __global__ void __launch_bounds__(256) select_count_kernel(const void* points, int dtype, int64_t n,
@@ -2181,10 +2184,11 @@ int b200icp_polar_to_cartesian(const double* raw, const int32_t* raw_len, int32_
 int b200icp_select_points(const void* points, int32_t dtype, int64_t n, int32_t mode, const double* key,
                           double cx, double cy, double threshold, void* out_points,
                           int64_t* count_out, int64_t* scratch, void* stream) {
-  if (!points || !out_points || !count_out || !scratch || n < 0) { set_error("select_points: bad arguments"); return B200ICP_ERR_INVALID_ARGUMENT; }
+  // an empty set may come with NULL points / out_points / key (an empty tensor has no storage)
+  if ((n > 0 && (!points || !out_points)) || !count_out || !scratch || n < 0) { set_error("select_points: bad arguments"); return B200ICP_ERR_INVALID_ARGUMENT; }
   if (dtype != B200ICP_F32 && dtype != B200ICP_F64) { set_error("select_points: bad dtype"); return B200ICP_ERR_INVALID_ARGUMENT; }
   if (mode != 0 && mode != 1) { set_error("select_points: mode must be 0 (key) or 1 (radius)"); return B200ICP_ERR_INVALID_ARGUMENT; }
-  if (mode == 0 && !key) { set_error("select_points: mode 0 needs key"); return B200ICP_ERR_INVALID_ARGUMENT; }
+  if (mode == 0 && !key && n > 0) { set_error("select_points: mode 0 needs key"); return B200ICP_ERR_INVALID_ARGUMENT; }
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int64_t blocks = (n + kSelBlock - 1) / kSelBlock;
   if (blocks > 0) {
@@ -2204,7 +2208,7 @@ int b200icp_select_points(const void* points, int32_t dtype, int64_t n, int32_t 
 }
 
 int b200icp_chain_poses(const double* poses, int64_t n, double* out, void* stream) {
-  if (!poses || !out || n < 0) { set_error("chain_poses: bad arguments"); return B200ICP_ERR_INVALID_ARGUMENT; }
+  if ((n > 0 && !poses) || !out || n < 0) { set_error("chain_poses: bad arguments"); return B200ICP_ERR_INVALID_ARGUMENT; }
   chain_poses_kernel<<<1, 1024, 0, reinterpret_cast<cudaStream_t>(stream)>>>(poses, n, out);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "chain_poses_kernel");

@@ -9,8 +9,11 @@
 // builds with lexsort.  Parity-unpinned against Open3D (not vendored by the reference): the
 // semantics are pinned by oracle.icp_oracle.voxel_down_sample_2d.
 //
-// keys (cell_y, cell_x) -> cub radix sort of (key, index) -> one thread per point: segment heads
-// average their run in the original point order (deterministic).
+// cells (cell_y, cell_x), int64 per axis -> two stable cub radix sorts of (key, index): by cell_x,
+// then by cell_y -> order (cell_y, cell_x, input order) -> one thread per point: segment heads
+// average their run in the original point order (deterministic).  Points whose cell is not an
+// int64 (non-finite coordinates, |p / voxel_size| >= 2^63) are skipped, as b200icp_occ_update
+// skips non-finite points.
 #include <cuda_runtime.h>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -23,33 +26,67 @@ void b200icp_set_error_str(const char* msg);
 
 namespace {
 
+// sort key of a skipped point: above every biased int64 cell (the largest cell of a double below
+// 2^63 is 2^63 - 1024), so skipped points sort last and never join a cell's run
+constexpr uint64_t kSkipKey = ~0ull;
+
 __device__ __forceinline__ double2 vx_load(const void* base, int dtype, int64_t i) {
   if (dtype == B200ICP_F64) return reinterpret_cast<const double2*>(base)[i];
   const float2 v = reinterpret_cast<const float2*>(base)[i];
   return make_double2((double)v.x, (double)v.y);
 }
 
-__global__ void voxel_key_kernel(const void* points, int dtype, int64_t n, double inv_voxel,
-                                 uint64_t* keys, int32_t* idx) {
+// cell = floor(p / voxel) (d.py:11-12), biased to unsigned so that the radix order is the signed
+// order; kSkipKey for both axes unless both cells are int64
+__device__ __forceinline__ void vx_cell(const void* points, int dtype, int64_t i, double inv_voxel,
+                                        uint64_t& kx, uint64_t& ky) {
+  const double2 q = vx_load(points, dtype, i);
+  const double fx = floor(q.x * inv_voxel), fy = floor(q.y * inv_voxel);
+  const double lim = 9223372036854775808.0;                 // 2^63
+  if (!(fabs(fx) < lim && fabs(fy) < lim)) { kx = ky = kSkipKey; return; }
+  kx = (uint64_t)(int64_t)fx ^ 0x8000000000000000ull;
+  ky = (uint64_t)(int64_t)fy ^ 0x8000000000000000ull;
+}
+
+__global__ void voxel_key_x_kernel(const void* points, int dtype, int64_t n, double inv_voxel,
+                                   uint64_t* keys, int32_t* idx) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const double2 q = vx_load(points, dtype, i);
-  // cell = floor(p / voxel) (d.py:11-12); biased to unsigned so the radix order is (cy, cx)
-  const int64_t gx = (int64_t)floor(q.x * inv_voxel), gy = (int64_t)floor(q.y * inv_voxel);
-  keys[i] = ((uint64_t)(uint32_t)((int32_t)gy ^ 0x80000000)) << 32 | (uint32_t)((int32_t)gx ^ 0x80000000);
+  uint64_t kx, ky;
+  vx_cell(points, dtype, i, inv_voxel, kx, ky);
+  keys[i] = kx;
   idx[i] = (int32_t)i;
 }
 
-__global__ void voxel_mean_kernel(const void* points, int dtype, int64_t n, const uint64_t* keys,
-                                  const int32_t* idx, int32_t* head_flag) {
+// cell_y of the points in cell_x order, for the second (stable) pass
+__global__ void voxel_key_y_kernel(const void* points, int dtype, int64_t n, double inv_voxel,
+                                   const int32_t* idx, uint64_t* keys) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  head_flag[i] = (i == 0 || keys[i] != keys[i - 1]) ? 1 : 0;
+  uint64_t kx, ky;
+  vx_cell(points, dtype, idx[i], inv_voxel, kx, ky);
+  keys[i] = ky;
 }
 
-// one thread per sorted position; heads walk their run (radix sort is stable, so a run lists its
+// head of a run: a kept point whose cell differs from its predecessor's in sorted order
+__global__ void voxel_head_kernel(const void* points, int dtype, int64_t n, double inv_voxel,
+                                  const uint64_t* keys_y, const int32_t* idx, int32_t* head_flag) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if (keys_y[i] == kSkipKey) { head_flag[i] = 0; return; }
+  int flag = 1;
+  if (i > 0) {
+    uint64_t ax, ay, bx, by;
+    vx_cell(points, dtype, idx[i], inv_voxel, ax, ay);
+    vx_cell(points, dtype, idx[i - 1], inv_voxel, bx, by);
+    flag = (ax != bx || ay != by) ? 1 : 0;
+  }
+  head_flag[i] = flag;
+}
+
+// one thread per sorted position; heads walk their run (both sorts are stable, so a run lists its
 // points in the original order) and write the mean to the slot given by the scanned head count
-__global__ void voxel_emit_kernel(const void* points, int dtype, int64_t n, const uint64_t* keys,
+__global__ void voxel_emit_kernel(const void* points, int dtype, int64_t n, const uint64_t* keys_y,
                                   const int32_t* idx, const int32_t* head_flag,
                                   const int32_t* head_rank, void* out, int64_t* count_out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -58,18 +95,18 @@ __global__ void voxel_emit_kernel(const void* points, int dtype, int64_t n, cons
   if (!head_flag[i]) return;
   double sx = 0.0, sy = 0.0;
   int64_t k = i;
-  const uint64_t key = keys[i];
-  for (; k < n && keys[k] == key; ++k) {
+  do {
     const double2 q = vx_load(points, dtype, idx[k]);
     sx += q.x; sy += q.y;
-  }
+    ++k;
+  } while (k < n && !head_flag[k] && keys_y[k] != kSkipKey);
   const double inv = 1.0 / (double)(k - i);
   const int64_t slot = head_rank[i];
   if (dtype == B200ICP_F64) reinterpret_cast<double2*>(out)[slot] = make_double2(sx * inv, sy * inv);
   else reinterpret_cast<float2*>(out)[slot] = make_float2((float)(sx * inv), (float)(sy * inv));
 }
 
-// inclusive scan of head flags minus one (single CTA; n is a scan, i.e. <= a few 10^5 points)
+// inclusive scan of head flags minus one (single CTA, a contiguous segment per thread)
 __global__ void __launch_bounds__(1024) voxel_scan_kernel(const int32_t* flag, int64_t n, int32_t* rank) {
   __shared__ int32_t tot[1024];
   const int tid = threadIdx.x;
@@ -155,14 +192,21 @@ int b200icp_voxel_downsample(const void* points, int32_t dtype, int64_t n, doubl
   int32_t* flags = reinterpret_cast<int32_t*>(base + w.flags);
   int32_t* rank = reinterpret_cast<int32_t*>(base + w.rank);
   const unsigned blocks = (unsigned)((n + 255) / 256);
-  voxel_key_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, 1.0 / voxel_size, keys_in, idx_in);
+  const double inv = 1.0 / voxel_size;
+  // pass 1 by cell_x: keys_in, idx_in -> keys_out, idx_out; pass 2 by cell_y of that order:
+  // keys_in, idx_out -> keys_out, idx_in.  Stable, so the result is (cell_y, cell_x, input order).
+  voxel_key_x_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, inv, keys_in, idx_in);
   size_t cub_bytes = w.cub_bytes;
   cudaError_t e = cub::DeviceRadixSort::SortPairs(base + w.cub, cub_bytes, keys_in, keys_out, idx_in, idx_out,
                                                   (int)n, 0, 64, st);
   if (e != cudaSuccess) return vfail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
-  voxel_mean_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, keys_out, idx_out, flags);
+  voxel_key_y_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, inv, idx_out, keys_in);
+  cub_bytes = w.cub_bytes;
+  e = cub::DeviceRadixSort::SortPairs(base + w.cub, cub_bytes, keys_in, keys_out, idx_out, idx_in, (int)n, 0, 64, st);
+  if (e != cudaSuccess) return vfail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
+  voxel_head_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, inv, keys_out, idx_in, flags);
   voxel_scan_kernel<<<1, 1024, 0, st>>>(flags, n, rank);
-  voxel_emit_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, keys_out, idx_out, flags, rank, out_points, count_out);
+  voxel_emit_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, keys_out, idx_in, flags, rank, out_points, count_out);
   e = cudaGetLastError();
   if (e != cudaSuccess) return vfail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
   return B200ICP_OK;

@@ -172,6 +172,8 @@ int b200icp_align_batch(const b200icp_problem* prob, int64_t n_pairs,
  * target, the first min(src_len, tgt_len) points of each pair).
  * Replaces best_fit_transform(A, B) (labels_segmentation/icp.py:5-26).
  *   pose_out [n_pairs][6] = R00 R01 R10 R11 tx ty.  Any pitch.  Degenerate H = 0 gives R = I.
+ *   The sums take each cloud relative to its own first point, so clouds far apart (1e6 mm, 1 mm
+ *   spread) keep the accuracy of clouds near the origin.
  */
 int b200icp_best_fit_batch(const b200icp_problem* prob, int64_t n_pairs, double* pose_out,
                            void* stream);
@@ -181,12 +183,15 @@ int b200icp_best_fit_batch(const b200icp_problem* prob, int64_t n_pairs, double*
  * polar -> Cartesian with order-preserving compaction.
  * Replaces polar_to_cartesian_3d (duc/ICP_LIDAR/process.py:38-52).
  *   raw      [n_scans][raw_pitch][3] float64 rows (quality, angle_deg, distance_mm)
- *   raw_len  [n_scans] valid rows per scan
+ *   raw_len  [n_scans] valid rows per scan (NULL = raw_pitch; values above raw_pitch read raw_pitch rows)
  *   filter   NULL = the canonical thresholds of process.py:45-46; the reference's other copies of
  *            the function differ only in these constants: slam_offline.py:68-69 (0 < d < 10000,
  *            q > 13, arc), realtime_2.py:160-161 (0 < d < 5000, q > 5, no arc), realtime_1.py:164-167
  *            and b.py:173-177 (as realtime_2 with y = +d sin)
  *   xy_out   [n_scans][out_pitch][2] float64;  len_out [n_scans]
+ *            The kept rows are written in input order.  A scan keeping more than out_pitch rows
+ *            yields its first out_pitch kept points and len_out = out_pitch; rows of xy_out past
+ *            len_out are zero.
  */
 typedef struct b200icp_polar_filter {
   double min_dist, max_dist;    /* keep min_dist < distance < max_dist   (process.py:46: 1000, 9000) */
@@ -314,8 +319,11 @@ int b200icp_peer_free(void* ptr);
  *           scan (b200icp_nn_batch / b200icp_s2m_search) and threshold = d^2 this replaces
  *           remove_dynamic_points (duc/ICP_LIDAR/process.py:75-84: distances < distance_threshold).
  *   mode 1: keep point i iff |p_i - (cx, cy)|^2 < threshold: the local-map radius crop
- *           (duc/ICP_LIDAR/mainn.py:300-303: distances_sq < LOCAL_MAP_RADIUS_MM**2).
+ *           (duc/ICP_LIDAR/mainn.py:300-303: distances_sq < LOCAL_MAP_RADIUS_MM**2).  The squared
+ *           distance is rounded as NumPy rounds it, (x - cx)^2 and (y - cy)^2 each rounded before
+ *           the add (no FMA), so the kept set equals NumPy's bit for bit, on the circle too.
  * out_points [n][2] (same dtype), count_out: device int64, scratch: device int64[ceil(n/1024)+1].
+ * n = 0 writes count_out = 0; points, key and out_points may then be NULL.
  */
 int b200icp_select_points(const void* points, int32_t dtype, int64_t n, int32_t mode,
                           const double* key, double cx, double cy, double threshold,
@@ -325,7 +333,8 @@ int b200icp_select_points(const void* points, int32_t dtype, int64_t n, int32_t 
  * Sequence odometry: prefix composition of the pairwise poses of consecutive scans into global
  * poses, out[0] = identity, out[k+1] = out[k] o poses[k]  (the frame-to-frame pose carry of the
  * reference's SLAM loops, duc/ICP_LIDAR/slam_offline.py:382-392).
- *   poses [n][6], out [n+1][6], both R00 R01 R10 R11 tx ty, float64, device.
+ *   poses [n][6], out [n+1][6], both R00 R01 R10 R11 tx ty, float64, device.  n = 0 writes the
+ *   identity to out[0]; poses may then be NULL.
  */
 int b200icp_chain_poses(const double* poses, int64_t n, double* out, void* stream);
 
@@ -336,6 +345,9 @@ int b200icp_chain_poses(const double* poses, int64_t n, double* out, void* strea
  * (duc/ICP_LIDAR/gicp_lidar.py:8-11,20-21) and for duplicate removal (process.py:68-73); the 2D
  * grid is labels_segmentation/d.py:10-16.  Parity-unpinned against Open3D (output order of
  * Open3D is unspecified).  out_points [n][2] (same dtype), count_out device int64.
+ * Cells are int64 per axis, so cells 2^32 apart stay apart.  Points whose cell is not an int64
+ * (non-finite coordinates, |p / voxel_size| >= 2^63) are skipped, like the non-finite points of
+ * b200icp_occ_update; when every point is skipped, count_out = 0.
  */
 int64_t b200icp_voxel_workspace_bytes(int64_t n);
 int b200icp_voxel_downsample(const void* points, int32_t dtype, int64_t n, double voxel_size,

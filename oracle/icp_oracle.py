@@ -392,22 +392,24 @@ def synth_trajectory_scans(n_scans, n_points=360, seed=4096, dtype=np.float32):
 # ----------------------------------------------------------------------------
 def voxel_down_sample_2d(points, voxel_size):
     """One point per occupied cell floor(p / voxel_size): the mean of its points, cells ordered by
-    (cell_y, cell_x).  PARITY-UNPINNED against Open3D (not vendored; its output order is the
-    iteration order of a hash map); this function is the definition the CUDA path is held to."""
+    (cell_y, cell_x), int64 per axis.  Points whose cell is not an int64 (non-finite coordinates,
+    |p / voxel_size| >= 2^63) are skipped.  PARITY-UNPINNED against Open3D (not vendored; its output
+    order is the iteration order of a hash map); this function is the definition the CUDA path is
+    held to."""
     p = np.asarray(points, dtype=np.float64)[:, :2]
+    inv = 1.0 / float(voxel_size)
+    f = np.floor(p * inv)
+    keep = np.all(np.abs(f) < 2.0 ** 63, axis=1)
+    p, f = p[keep], f[keep]
     if len(p) == 0:
         return p.copy()
-    inv = 1.0 / float(voxel_size)
-    gx = np.floor(p[:, 0] * inv).astype(np.int64)
-    gy = np.floor(p[:, 1] * inv).astype(np.int64)
+    gx, gy = f[:, 0].astype(np.int64), f[:, 1].astype(np.int64)
     order = np.lexsort((np.arange(len(p)), gx, gy))            # stable: (gy, gx), then input order
     gxs, gys = gx[order], gy[order]
     head = np.ones(len(p), dtype=bool)
     head[1:] = (gxs[1:] != gxs[:-1]) | (gys[1:] != gys[:-1])
     seg = np.cumsum(head) - 1
     out = np.zeros((seg[-1] + 1, 2))
-    cnt = np.zeros(seg[-1] + 1)
-    for q in range(len(p)):                                    # sequential sums, input order per cell
-        out[seg[q]] += p[order[q]]
-        cnt[seg[q]] += 1.0
+    cnt = np.bincount(seg).astype(np.float64)
+    np.add.at(out, seg, p[order])                              # unbuffered, in index order: sequential
     return out * (1.0 / cnt)[:, None]
