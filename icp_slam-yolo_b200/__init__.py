@@ -10,6 +10,7 @@ from .icp import (IcpOutput, best_fit_transform, icp, icp_full, nearest_neighbor
 from .registration import (AlignResult, ScanTable, align_pairs, alloc_outputs,   # noqa: F401
                            best_fit, ffma_probe, nn_search, polar_to_cartesian)
 from .odometry import align_consecutive, chain_poses         # noqa: F401
+from .gicp import estimate_covariances, gicp_consecutive, gicp_pairs, registration_gicp   # noqa: F401
 from .sharding import shard_range, triangle_pair, triangle_pair_count   # noqa: F401
 from .scan_to_map import MapShard, ScanToMap, ScanToMapResult, scan_to_map_icp   # noqa: F401
 from .mapping import crop_local_map, remove_dynamic_points, voxel_down_sample   # noqa: F401
@@ -24,4 +25,5 @@ __all__ = [
     "triangle_pair", "triangle_pair_count", "scan_io", "MapShard", "ScanToMap", "ScanToMapResult",
     "scan_to_map_icp", "crop_local_map", "remove_dynamic_points", "voxel_down_sample",
     "OccupancyGrid", "map_io", "hostmem", "OfflineSlam", "SlamConfig",
+    "estimate_covariances", "gicp_pairs", "gicp_consecutive", "registration_gicp",
 ]

@@ -53,6 +53,14 @@ class Outputs(C.Structure):
     ]
 
 
+class GicpOptions(C.Structure):
+    _fields_ = [
+        ("max_iterations", C.c_int32), ("reserved", C.c_int32),
+        ("max_corr_dist", C.c_double), ("relative_fitness", C.c_double), ("relative_rmse", C.c_double),
+        ("init_pose", C.c_void_p),
+    ]
+
+
 class PolarFilter(C.Structure):
     _fields_ = [
         ("min_dist", C.c_double), ("max_dist", C.c_double), ("min_quality", C.c_double),
@@ -95,6 +103,10 @@ SYMBOLS = {
     "b200icp_nn_batch": (C.c_int, [C.POINTER(Problem), C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "b200icp_align_batch": (C.c_int, [C.POINTER(Problem), C.c_int64, C.POINTER(Options),
                                       C.POINTER(Outputs), C.c_void_p]),
+    "b200icp_estimate_covariances": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                               C.c_double, C.c_void_p, C.c_void_p]),
+    "b200icp_gicp_batch": (C.c_int, [C.POINTER(Problem), C.c_int64, C.POINTER(GicpOptions), C.c_void_p, C.c_void_p,
+                                     C.POINTER(Outputs), C.c_void_p]),
     "b200icp_best_fit_batch": (C.c_int, [C.POINTER(Problem), C.c_int64, C.c_void_p, C.c_void_p]),
     "b200icp_polar_to_cartesian": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),

@@ -3,8 +3,9 @@
 Mirrors ``duc/ICP_LIDAR/slam_offline.py:318-455`` step by step -- same order, same thresholds
 (``Config.py``), same early ``continue`` on a rejected registration -- with one substitution: the
 registration call ``gicp(points, local_map, threshold, voxel, trans_init)`` (Open3D Generalized
-ICP, slam_offline.py:108-144,382) is the point-to-point loop of ``labels_segmentation/icp.py:28-53``
-behind the same call shape (``registration_p2p``).  Open3D is not vendored by the reference, so the
+ICP, slam_offline.py:108-144,382) is, by default, the point-to-point loop of
+``labels_segmentation/icp.py:28-53`` behind the same call shape (``registration_p2p``);
+``SlamConfig(registration="gicp")`` selects the 2D Generalized ICP of ``gicp.py`` instead.  Open3D is not vendored by the reference, so the
 loop as a whole is parity-UNPINNED; every step in it is pinned on its own (DESIGN.md §2), and
 ``tests/test_slam_gpu.py`` replays it against the same composition of the CPU oracles.
 
@@ -21,6 +22,7 @@ import numpy as np
 import torch
 
 from . import map_io
+from .gicp import registration_gicp
 from .icp import registration_p2p
 from .mapping import crop_local_map, remove_dynamic_points, voxel_down_sample
 from .occupancy import OccupancyGrid
@@ -42,6 +44,7 @@ class SlamConfig:
     min_scan_points: int = 10                           # slam_offline.py:353
     max_iteration: int = 50                             # gicp_lidar.py:27 (ICPConvergenceCriteria)
     tolerance: float = 1e-5
+    registration: str = "p2p"                           # "p2p" (registration_p2p) or "gicp" (registration_gicp)
 
     @property
     def map_width_pixels(self) -> int:
@@ -72,6 +75,8 @@ class OfflineSlam:
 
     def __post_init__(self):
         c = self.config
+        if c.registration not in ("p2p", "gicp"):
+            raise ValueError(f"SlamConfig.registration must be 'p2p' or 'gicp', got {c.registration!r}")
         self.map_center_px = (c.map_width_pixels // 2, c.map_height_pixels // 2)          # :320
         self.grid = OccupancyGrid(c.map_height_pixels, c.map_width_pixels, self.map_center_px,
                                   c.resolution_mm_per_pixel, device=self.device)           # :319
@@ -112,9 +117,13 @@ class OfflineSlam:
             map_for_icp = crop_local_map(self.global_map, robot[:2], c.local_map_radius_mm, c.min_icp_map_points)
         else:
             map_for_icp = self.global_map
-        rmse, T = registration_p2p(current_points, map_for_icp, c.icp_threshold, c.icp_voxel_size,
-                                   trans_init=self.global_pose, max_iteration=c.max_iteration,
-                                   tolerance=c.tolerance)                                   # :382
+        if c.registration == "gicp":                                                       # :382
+            rmse, T = registration_gicp(current_points, map_for_icp, c.icp_threshold, c.icp_voxel_size,
+                                        trans_init=self.global_pose, max_iteration=c.max_iteration)
+        else:
+            rmse, T = registration_p2p(current_points, map_for_icp, c.icp_threshold, c.icp_voxel_size,
+                                       trans_init=self.global_pose, max_iteration=c.max_iteration,
+                                       tolerance=c.tolerance)
         if rmse > c.max_rmse_threshold:                                                     # :386-387: `continue`
             return FrameResult(False, float(rmse), self.global_pose.copy(), int(self.global_map.shape[0]))
         self.global_pose = T                                                                # :390

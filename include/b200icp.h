@@ -168,6 +168,59 @@ int b200icp_align_batch(const b200icp_problem* prob, int64_t n_pairs,
                         void* stream);
 
 /*
+ * 2D Generalized ICP (line-to-line), the registration objective of the reference's
+ * gicp(points1, points2, threshold, voxel, trans_init) (duc/ICP_LIDAR/gicp_lidar.py:12-36, called at
+ * slam_offline.py:382 and mainn.py:311).  Open3D is not vendored, so the model is defined by
+ * oracle/gicp_oracle.py (parity-unpinned; DESIGN.md 4.8).
+ *
+ * b200icp_estimate_covariances: per point of every row of a table, the k nearest points of the same
+ * row under the order (d^2, index) (the point itself included; all of them when the row has fewer
+ * than k), their population covariance C (sums taken sequentially in that order, no contraction)
+ * and the regularised  C_reg = u u^T + epsilon (I - u u^T),  u = (cos phi, sin phi),
+ * phi = atan2(2 cxy, cxx - cyy) / 2.  C_reg = I when fewer than 3 neighbours or cxx + cyy = 0.
+ *   points  [rows][pitch][2] (dtype);  len [rows] valid points per row (NULL = pitch)
+ *   cov_out [rows][pitch][3] float64 (cxx, cxy, cyy); entries past len are 0.
+ *   3 <= k <= 32; epsilon finite and > 0; pitch <= 65536 (O(n^2) per row: local maps and scans,
+ *   not the scan-to-map map).
+ */
+int b200icp_estimate_covariances(const void* points, const int32_t* len, int32_t rows, int32_t pitch,
+                                 int32_t dtype, int32_t k, double epsilon, double* cov_out, void* stream);
+
+typedef struct b200icp_gicp_options {
+  int32_t max_iterations;   /* updates (gicp_lidar.py:27: 50)                                   */
+  int32_t reserved;
+  double max_corr_dist;     /* <= 0 or +inf: no gate; else keep pairs with distance < it        */
+  double relative_fitness;  /* stop when |d fitness| < relative_fitness AND                     */
+  double relative_rmse;     /*           |d rmse| < relative_rmse (Open3D's defaults: 1e-6)    */
+  const double* init_pose;  /* NULL or [n_pairs][6] = R00 R01 R10 R11 tx ty                     */
+} b200icp_gicp_options;
+
+/*
+ * Whole GICP loop per pair, one CTA per pair (Open3D's RegistrationICP shape): evaluate at the
+ * initial pose; then per update one float64 Gauss-Newton step in (dtheta, dx, dy) about the pivot
+ * c = current pose applied to the centroid of the original source, with
+ *   J = [[-(s_y - c_y), 1, 0], [s_x - c_x, 0, 1]],  r = b - s,  M = (C^B_j + R C^A_i R^T)^-1,
+ *   H = sum J^T M J,  g = sum J^T M r,  H x = g by a 3x3 Cholesky factorisation;
+ * apply s <- R(dtheta)(s - c) + c + dt and T <- dT o T (as increments: s + ((R(dtheta) - I)(s - c) + dt),
+ * so a zero step changes nothing), and evaluate again.  An evaluation takes the
+ * exact float64 nearest target of every source point (lowest index on ties, as b200icp_nn_batch),
+ * the gate of b200icp_align_batch, fitness = inliers / n and rmse = sqrt(mean d^2) over inliers.
+ * Stops when both relative criteria hold, after max_iterations updates, when an evaluation has
+ * no inlier (error = rmse = +inf) or when a Cholesky pivot is not finite and positive (no update).
+ * n = 0 or m = 0: the initial pose, iterations = 0, error = rmse = +inf.
+ *   src_cov / tgt_cov: [rows][pitch][3] from b200icp_estimate_covariances, laid out like the point
+ *   tables and indexed by the same rows (ROWWISE odometry offsets src_cov by one row, like
+ *   src_points).  src_pitch <= 1024; tgt_pitch <= 65536 (targets are searched in shared-memory
+ *   tiles of 4,096 and the results merged exactly).
+ *   Outputs (b200icp_outputs): pose_total; pose_last = the last applied increment; error = mean
+ *   inlier distance, rmse, inliers and indices at the FINAL pose; iterations = applied updates;
+ *   index_history[it] = the correspondences update `it` used; evaluated_pairs unused (may be NULL).
+ */
+int b200icp_gicp_batch(const b200icp_problem* prob, int64_t n_pairs, const b200icp_gicp_options* opt,
+                       const double* src_cov, const double* tgt_cov, const b200icp_outputs* out,
+                       void* stream);
+
+/*
  * Least-squares rigid transform between MATCHED rows (row i of the source onto row i of the
  * target, the first min(src_len, tgt_len) points of each pair).
  * Replaces best_fit_transform(A, B) (labels_segmentation/icp.py:5-26).
