@@ -27,13 +27,11 @@
 #include <cstdint>
 #include <cstdio>
 
-#include "b200icp.h"
-
-void b200icp_set_error_str(const char* msg);
+#include "common.cuh"
+#include "compact.cuh"
 
 namespace {
 
-constexpr unsigned kFullMask = 0xffffffffu;
 constexpr int kOccThreads = 512;
 constexpr int kOccUnroll = 5;                 // on-map fallback: 5 x 32 cells per trip
 constexpr int kOccTileCells = 54 * 1024;      // float32 map cells held in shared memory (216 KB)
@@ -42,13 +40,6 @@ constexpr int kOccSmemBytes = 227 * 1024;     // tile + ring of per-ray cell lis
 constexpr int kOccGroup = 512;                // rays whose end cells are resident at once
 constexpr int kOccMaxSlots = 16;              // ring slots (rays expanded ahead of the ordered loop)
 constexpr int kOccProducers = 12;             // warps expanding rays into the ring
-
-cudaError_t occ_fail(cudaError_t e, const char* what) {
-  char buf[256];
-  snprintf(buf, sizeof(buf), "%s: %s", what, cudaGetErrorString(e));
-  b200icp_set_error_str(buf);
-  return e;
-}
 
 // int(): truncation toward zero (Python's int(float)); callers test finiteness first
 __device__ __forceinline__ long long py_int(double v) { return (long long)v; }
@@ -137,7 +128,7 @@ __device__ __forceinline__ void occ_cast_ray(float* mem, int L, int lane, float 
     for (int u = 0; u < kOccUnroll; ++u) {
       const int k = k0 + u * 32 + lane;
       const bool free_cell = off[u] >= 0 && k < L;
-      const unsigned hit = __ballot_sync(kFullMask, free_cell && v[u] >= thr_up);                 // :165
+      const unsigned hit = __ballot_sync(kFull, free_cell && v[u] >= thr_up);                 // :165
       if (!stopped) {
         const int first = hit ? __ffs(hit) - 1 : 32;
         if (free_cell && lane < first) {
@@ -381,9 +372,9 @@ __global__ void __launch_bounds__(kOccThreads) occ_update_kernel(b200icp_occ_gri
           }
           ends[b] = e;
         }
-        mnx = __reduce_min_sync(kFullMask, mnx); mxx = __reduce_max_sync(kFullMask, mxx);
-        mny = __reduce_min_sync(kFullMask, mny); mxy = __reduce_max_sync(kFullMask, mxy);
-        unlisted = __reduce_max_sync(kFullMask, unlisted);
+        mnx = __reduce_min_sync(kFull, mnx); mxx = __reduce_max_sync(kFull, mxx);
+        mny = __reduce_min_sync(kFull, mny); mxy = __reduce_max_sync(kFull, mxy);
+        unlisted = __reduce_max_sync(kFull, unlisted);
         if (lane == 0 && mxx >= 0) {
           atomicMin(&ctrl[20], mnx); atomicMax(&ctrl[21], mxx); atomicMin(&ctrl[22], mny); atomicMax(&ctrl[23], mxy);
           if (unlisted) atomicMax(&ctrl[25], 1);
@@ -561,9 +552,9 @@ __global__ void __launch_bounds__(kOccThreads) occ_update_kernel(b200icp_occ_gri
                   }
                   const bool h0 = v0 >= thr_up, h1 = v1 >= thr_up, h2 = v2 >= thr_up, h3 = v3 >= thr_up;   // :165
                   int first = 4;                                            // cells of this lane to update
-                  if (__any_sync(kFullMask, h0 | h1 | h2 | h3)) {          // :166 break
+                  if (__any_sync(kFull, h0 | h1 | h2 | h3)) {          // :166 break
                     const int mine = h0 ? 0 : h1 ? 1 : h2 ? 2 : h3 ? 3 : 4;
-                    const unsigned lanes = __ballot_sync(kFullMask, mine < 4);
+                    const unsigned lanes = __ballot_sync(kFull, mine < 4);
                     const int fl = __ffs(lanes) - 1;                        // first blocking lane
                     first = lane < fl ? 4 : lane == fl ? mine : 0;
                     stopped = true;
@@ -608,106 +599,30 @@ __global__ void __launch_bounds__(kOccThreads) occ_update_kernel(b200icp_occ_gri
 }
 
 // ---- point filter (process.py:203-249): keep iff outside the grid or probs[py, px] >= thr -------
-constexpr int kFiltBlock = 1024;
-
 template <typename T>
-__device__ __forceinline__ bool occ_keep(const T* points, int cols, int64_t i, const float* probs, int h, int w,
-                                         double cx, double cy, double res, float thr) {
-  const double fx = __dadd_rn(cx, __ddiv_rn((double)points[i * cols], res));          // :213
-  const double fy = __dsub_rn(cy, __ddiv_rn((double)points[i * cols + 1], res));      // :214
-  if (!(isfinite(fx) && isfinite(fy))) return true;
-  const long long px = py_int(fx), py = py_int(fy);
-  if (!(0 <= px && px < w && 0 <= py && py < h)) return true;                           // :216-218
-  return !(probs[py * w + px] < thr);                                                   // :220-221
-}
+struct OccKeep {
+  const T* points;
+  int cols;
+  const float* probs;
+  int h, w;
+  double cx, cy, res;
+  float thr;
+  __device__ __forceinline__ bool operator()(int64_t i) const {
+    const double fx = __dadd_rn(cx, __ddiv_rn((double)points[i * cols], res));          // :213
+    const double fy = __dsub_rn(cy, __ddiv_rn((double)points[i * cols + 1], res));      // :214
+    if (!(isfinite(fx) && isfinite(fy))) return true;
+    const long long px = py_int(fx), py = py_int(fy);
+    if (!(0 <= px && px < w && 0 <= py && py < h)) return true;                           // :216-218
+    return !(probs[py * w + px] < thr);                                                   // :220-221
+  }
+};
 
-template <typename T>
-__global__ void __launch_bounds__(256) occ_filter_count_kernel(const T* points, int cols, int64_t n,
-                                                               const float* probs, int h, int w, double cx,
-                                                               double cy, double res, float thr,
-                                                               int64_t* block_counts) {
-  __shared__ int wc[8];
-  const int64_t base = (int64_t)blockIdx.x * kFiltBlock;
-  int c = 0;
-  for (int k = 0; k < 4; ++k) {
-    const int64_t i = base + k * 256 + threadIdx.x;
-    if (i < n && occ_keep(points, cols, i, probs, h, w, cx, cy, res, thr)) ++c;
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(kFullMask, c, o);
-  if ((threadIdx.x & 31) == 0) wc[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int t = 0;
-    for (int q = 0; q < 8; ++q) t += wc[q];
-    block_counts[blockIdx.x] = t;
-  }
-}
-
-// exclusive scan of the per-block counts in place (one CTA; see select_scan_kernel in b200icp.cu)
-__global__ void __launch_bounds__(1024) occ_filter_scan_kernel(int64_t* counts, int64_t n_blocks, int64_t* count_out) {
-  __shared__ long long wsum[32];
-  const unsigned full = 0xffffffffu;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t per = (n_blocks + 1023) / 1024;
-  const int64_t b = min(n_blocks, tid * per), e = min(n_blocks, b + per);
-  long long s = 0;
-  for (int64_t k = b; k < e; ++k) s += counts[k];
-  long long inc = s;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const long long v = __shfl_up_sync(full, inc, o);
-    if (lane >= o) inc += v;
-  }
-  if (lane == 31) wsum[warp] = inc;
-  __syncthreads();
-  if (warp == 0) {
-    const long long w = wsum[lane];
-    long long winc = w;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const long long v = __shfl_up_sync(full, winc, o);
-      if (lane >= o) winc += v;
-    }
-    wsum[lane] = winc - w;
-  }
-  __syncthreads();
-  long long run = wsum[warp] + inc - s;
-  for (int64_t k = b; k < e; ++k) { const long long c = counts[k]; counts[k] = run; run += c; }
-  if (tid == 1023) *count_out = run;
-}
-
-template <typename T>
-__global__ void __launch_bounds__(256) occ_filter_scatter_kernel(const T* points, int cols, int64_t n,
-                                                                 const float* probs, int h, int w, double cx,
-                                                                 double cy, double res, float thr,
-                                                                 const int64_t* block_offsets,
-                                                                 int64_t* kept_index) {
-  __shared__ int wc[4][8];
-  const int64_t base = (int64_t)blockIdx.x * kFiltBlock;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  bool keep[4];
-  unsigned ballots[4];
-  for (int k = 0; k < 4; ++k) {
-    const int64_t i = base + k * 256 + threadIdx.x;
-    keep[k] = i < n && occ_keep(points, cols, i, probs, h, w, cx, cy, res, thr);
-    ballots[k] = __ballot_sync(kFullMask, keep[k]);
-    if (lane == 0) wc[k][warp] = __popc(ballots[k]);
-  }
-  __syncthreads();
-  int64_t off = block_offsets[blockIdx.x];
-  for (int k = 0; k < 4; ++k) {
-    int before = 0;
-    for (int q = 0; q < warp; ++q) before += wc[k][q];
-    if (keep[k]) kept_index[off + before + __popc(ballots[k] & ((1u << lane) - 1u))] = base + k * 256 + threadIdx.x;
-    int row = 0;
-    for (int q = 0; q < 8; ++q) row += wc[k][q];
-    off += row;
-  }
-}
+struct KeptIndex {
+  int64_t* out;
+  __device__ __forceinline__ void operator()(int64_t dst, int64_t i) const { out[dst] = i; }
+};
 
 bool occ_grid_ok(const b200icp_occ_grid* g, const char* who) {
-  char buf[160];
   const char* why = nullptr;
   if (!g) why = "grid is NULL";
   else if (!g->probs) why = "grid.probs is NULL";
@@ -715,8 +630,7 @@ bool occ_grid_ok(const b200icp_occ_grid* g, const char* who) {
   else if (!(g->resolution > 0.0)) why = "grid.resolution must be > 0";
   else if (!(g->threshold_up > 0.0f)) why = "grid.threshold_up must be > 0";
   if (!why) return true;
-  snprintf(buf, sizeof(buf), "%s: %s", who, why);
-  b200icp_set_error_str(buf);
+  set_error(B200ICP_ERR_INVALID_ARGUMENT, "%s: %s", who, why);
   return false;
 }
 
@@ -728,12 +642,10 @@ int b200icp_occ_update(const b200icp_occ_grid* grid, int32_t n_maps, const void*
                        const int32_t* len, const double* robot_xy, int32_t n_frames, int32_t pitch,
                        void* stream) {
   if (!occ_grid_ok(grid, "occ_update")) return B200ICP_ERR_INVALID_ARGUMENT;
-  if (n_maps < 0 || n_frames < 0 || pitch < 0 || (!points && pitch > 0) || !robot_xy) {
-    b200icp_set_error_str("occ_update: bad arguments");
-    return B200ICP_ERR_INVALID_ARGUMENT;
-  }
-  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) { b200icp_set_error_str("occ_update: bad dtype"); return B200ICP_ERR_INVALID_ARGUMENT; }
-  if (grid->area < 0 || grid->area > 10000) { b200icp_set_error_str("occ_update: area must be in [0, 10000]"); return B200ICP_ERR_UNSUPPORTED_SHAPE; }
+  if (n_maps < 0 || n_frames < 0 || pitch < 0 || (!points && pitch > 0) || !robot_xy)
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "occ_update: bad arguments");
+  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "occ_update: bad dtype");
+  if (grid->area < 0 || grid->area > 10000) return set_error(B200ICP_ERR_UNSUPPORTED_SHAPE, "occ_update: area must be in [0, 10000]");
   if (n_maps == 0 || n_frames == 0 || pitch == 0) return B200ICP_OK;
   // ring of K cell lists behind the tile; a ray has <= area + 1 cells (int4 rows)
   int stride = (grid->area + 1 + 3) & ~3;
@@ -746,17 +658,15 @@ int b200icp_occ_update(const b200icp_occ_grid* grid, int32_t n_maps, const void*
   static thread_local int configured_device = -1;
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) { occ_fail(e, "occ_update: cudaGetDevice"); return B200ICP_ERR_CUDA; }
+  if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "occ_update: cudaGetDevice: %s", cudaGetErrorString(e));
   if (configured_device != dev) {
     e = cudaFuncSetAttribute(occ_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kOccSmemBytes);
-    if (e != cudaSuccess) { occ_fail(e, "occ_update: cudaFuncSetAttribute"); return B200ICP_ERR_CUDA; }
+    if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "occ_update: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     configured_device = dev;
   }
   occ_update_kernel<<<n_maps, kOccThreads, smem, reinterpret_cast<cudaStream_t>(stream)>>>(
       *grid, points, dtype, len, robot_xy, n_frames, pitch, K, stride);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) { occ_fail(e, "occ_update_kernel"); return B200ICP_ERR_CUDA; }
-  return B200ICP_OK;
+  return check_launch("occ_update_kernel");
 }
 
 int b200icp_occ_filter_points(const void* points, int32_t dtype, int32_t cols, int64_t n, const float* probs,
@@ -764,34 +674,17 @@ int b200icp_occ_filter_points(const void* points, int32_t dtype, int32_t cols, i
                               float free_threshold, int64_t* kept_index, int64_t* count_out,
                               int64_t* scratch, void* stream) {
   if (!points || !probs || !kept_index || !count_out || !scratch || n < 0 || h < 1 || w < 1 || cols < 2 ||
-      !(resolution > 0.0)) {
-    b200icp_set_error_str("occ_filter_points: bad arguments");
-    return B200ICP_ERR_INVALID_ARGUMENT;
-  }
-  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) { b200icp_set_error_str("occ_filter_points: bad dtype"); return B200ICP_ERR_INVALID_ARGUMENT; }
+      !(resolution > 0.0))
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "occ_filter_points: bad arguments");
+  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "occ_filter_points: bad dtype");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int64_t blocks = (n + kFiltBlock - 1) / kFiltBlock;
-  cudaError_t e;
-  if (blocks > 0) {
-    if (dtype == B200ICP_F64)
-      occ_filter_count_kernel<double><<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const double*>(points), cols, n, probs, h, w, center_x, center_y, resolution, free_threshold, scratch);
-    else
-      occ_filter_count_kernel<float><<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const float*>(points), cols, n, probs, h, w, center_x, center_y, resolution, free_threshold, scratch);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) { occ_fail(e, "occ_filter_count_kernel"); return B200ICP_ERR_CUDA; }
-  }
-  occ_filter_scan_kernel<<<1, 1024, 0, st>>>(scratch, blocks, count_out);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) { occ_fail(e, "occ_filter_scan_kernel"); return B200ICP_ERR_CUDA; }
-  if (blocks > 0) {
-    if (dtype == B200ICP_F64)
-      occ_filter_scatter_kernel<double><<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const double*>(points), cols, n, probs, h, w, center_x, center_y, resolution, free_threshold, scratch, kept_index);
-    else
-      occ_filter_scatter_kernel<float><<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const float*>(points), cols, n, probs, h, w, center_x, center_y, resolution, free_threshold, scratch, kept_index);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) { occ_fail(e, "occ_filter_scatter_kernel"); return B200ICP_ERR_CUDA; }
-  }
-  return B200ICP_OK;
+  if (dtype == B200ICP_F64)
+    return compact(OccKeep<double>{reinterpret_cast<const double*>(points), cols, probs, h, w, center_x, center_y,
+                                   resolution, free_threshold},
+                   KeptIndex{kept_index}, n, scratch, count_out, st, "occ_filter");
+  return compact(OccKeep<float>{reinterpret_cast<const float*>(points), cols, probs, h, w, center_x, center_y,
+                                resolution, free_threshold},
+                 KeptIndex{kept_index}, n, scratch, count_out, st, "occ_filter");
 }
 
 }  // extern "C"

@@ -1,6 +1,6 @@
 // scan2map.cu -- scan-to-map ICP against a large map sharded across GPUs (sm_100a).
 //
-// Same reference loop as b200icp.cu (labels_segmentation/icp.py:28-53) with a target set of
+// Same reference loop as the pair kernels (labels_segmentation/icp.py:28-53) with a target set of
 // millions of points, for the scan-to-local-map call shape of duc/ICP_LIDAR/mainn.py:297-318.
 //
 // Round-2 design: EXACT CULLING + EXACT SCAN, two launches per iteration.
@@ -46,9 +46,7 @@
 #include <cstdio>
 #include <cstring>
 
-#include "b200icp.h"
-
-void b200icp_set_error_str(const char* msg);   // defined in b200icp.cu
+#include "common.cuh"
 
 namespace {
 
@@ -60,7 +58,6 @@ constexpr int kSearchMinCtas = 4;     // 64 registers: 32 resident warps per SM 
 constexpr int kUpdateThreads = 256;
 constexpr int kMaxUpdateCtas = 64;
 constexpr int kMaxWorld = 32;
-constexpr unsigned kFull = 0xffffffffu;
 constexpr double kUp = 1.000000000001;     // rounds a computed float64 bound outwards
 constexpr double kDown = 0.999999999999;
 constexpr long long kNoIndex = 0x7fffffffffffffffLL;
@@ -73,18 +70,6 @@ struct Circle {           // 32 bytes: one entry of the chunk / super-chunk tabl
 // scratch words (uint32) at the start of the caller's scratch buffer; zeroed once by the caller,
 // every kernel leaves its ticket at 0
 enum { kTicketSearch = 0, kTicketUpdate = 1, kTicketFinish = 2, kScratchHeader = 64 };
-
-__device__ __forceinline__ double2 load_point(const void* base, int dtype, int64_t i) {
-  if (dtype == B200ICP_F64) return __ldg(reinterpret_cast<const double2*>(base) + i);
-  const float2 v = __ldg(reinterpret_cast<const float2*>(base) + i);
-  return make_double2((double)v.x, (double)v.y);
-}
-
-// float64 squared distance in NumPy's operation order (no contraction)
-__device__ __forceinline__ double dist2_f64(double sx, double sy, double2 t) {
-  const double dx = __dsub_rn(sx, t.x), dy = __dsub_rn(sy, t.y);
-  return __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
-}
 
 __device__ __forceinline__ Circle load_circle(const double* table, int64_t k) {
   const double2 a = __ldg(reinterpret_cast<const double2*>(table) + 2 * k);
@@ -907,20 +892,6 @@ __global__ void __launch_bounds__(256) s2m_finish_kernel(double* src64, int n, b
   }
 }
 
-int fail(const char* msg, int code) {
-  b200icp_set_error_str(msg);
-  return code;
-}
-
-int cuda_check(const char* what) {
-  cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) return B200ICP_OK;
-  char buf[256];
-  snprintf(buf, sizeof(buf), "%s: %s", what, cudaGetErrorString(e));
-  b200icp_set_error_str(buf);
-  return B200ICP_ERR_CUDA;
-}
-
 int update_ctas(int n) {
   const int c = (n + kUpdateThreads - 1) / kUpdateThreads;
   return c < 1 ? 1 : (c > kMaxUpdateCtas ? kMaxUpdateCtas : c);
@@ -956,55 +927,55 @@ int64_t b200icp_s2m_prepare_workspace_bytes(int64_t m) {
 int b200icp_s2m_prepare_map(const b200icp_s2m_shard* shard, void* workspace, int64_t workspace_bytes,
                             void* stream) {
   if (!shard || !shard->points || !shard->chunk_circle || !shard->super_circle)
-    return fail("s2m_prepare_map: NULL pointer", B200ICP_ERR_INVALID_ARGUMENT);
-  if (shard->m < 1) return fail("s2m_prepare_map: empty shard", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: NULL pointer");
+  if (shard->m < 1) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: empty shard");
   if (shard->dtype != B200ICP_F32 && shard->dtype != B200ICP_F64)
-    return fail("s2m_prepare_map: bad dtype", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: bad dtype");
   if ((shard->sorted_points == nullptr) != (shard->order == nullptr))
-    return fail("s2m_prepare_map: sorted_points and order go together", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: sorted_points and order go together");
   const int64_t n_chunks = (shard->m + kChunk - 1) / kChunk;
   const int64_t padded = b200icp_s2m_padded_chunks(shard->m);
-  if (padded > (1LL << 24)) return fail("s2m_prepare_map: shard too large", B200ICP_ERR_UNSUPPORTED_SHAPE);
+  if (padded > (1LL << 24)) return set_error(B200ICP_ERR_UNSUPPORTED_SHAPE, "s2m_prepare_map: shard too large");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const void* scanned = shard->points;
   if (shard->sorted_points) {                   // Morton order (see above)
-    if (shard->m > 0x7fffffffLL) return fail("s2m_prepare_map: spatial sort needs m < 2^31", B200ICP_ERR_UNSUPPORTED_SHAPE);
+    if (shard->m > 0x7fffffffLL) return set_error(B200ICP_ERR_UNSUPPORTED_SHAPE, "s2m_prepare_map: spatial sort needs m < 2^31");
     const SortWs w = sort_layout(shard->m);
-    if (!workspace || workspace_bytes < w.total) return fail("s2m_prepare_map: workspace too small", B200ICP_ERR_INVALID_ARGUMENT);
+    if (!workspace || workspace_bytes < w.total) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: workspace too small");
     unsigned char* base = reinterpret_cast<unsigned char*>(workspace);
     unsigned long long* box = reinterpret_cast<unsigned long long*>(base + w.box);
     unsigned* keys_in = reinterpret_cast<unsigned*>(base + w.keys_in);
     unsigned* keys_out = reinterpret_cast<unsigned*>(base + w.keys_out);
     int32_t* idx_in = reinterpret_cast<int32_t*>(base + w.idx_in);
     if (cudaMemsetAsync(box, 0xff, 16, st) != cudaSuccess || cudaMemsetAsync(box + 2, 0, 16, st) != cudaSuccess)
-      return cuda_check("cudaMemsetAsync");
+      return check_launch("cudaMemsetAsync");
     const unsigned blocks = (unsigned)((shard->m + 255) / 256);
     s2m_bbox_kernel<<<blocks < 1184u ? blocks : 1184u, 256, 0, st>>>(shard->points, shard->dtype, shard->m, box);
     s2m_morton_kernel<<<blocks, 256, 0, st>>>(shard->points, shard->dtype, shard->m, box, keys_in, idx_in);
     size_t cub_bytes = w.cub_bytes;
     cudaError_t e = cub::DeviceRadixSort::SortPairs(base + w.cub, cub_bytes, keys_in, keys_out, idx_in, shard->order,
                                                     (int)shard->m, 0, 32, st);
-    if (e != cudaSuccess) return fail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
+    if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "%s", cudaGetErrorString(e));
     s2m_gather_kernel<<<blocks, 256, 0, st>>>(shard->points, shard->dtype, shard->m, shard->order, shard->sorted_points);
-    int rc = cuda_check("s2m spatial sort");
+    int rc = check_launch("s2m spatial sort");
     if (rc) return rc;
     scanned = shard->sorted_points;
   }
   s2m_prepare_kernel<<<(unsigned)padded, 256, 0, st>>>(scanned, shard->dtype, shard->m, (int)n_chunks,
                                                        shard->chunk_circle);
-  int rc = cuda_check("s2m_prepare_kernel");
+  int rc = check_launch("s2m_prepare_kernel");
   if (rc) return rc;
   s2m_super_kernel<<<(unsigned)(padded / kSuper), 32, 0, st>>>(shard->chunk_circle, shard->super_circle);
-  return cuda_check("s2m_super_kernel");
+  return check_launch("s2m_super_kernel");
 }
 
 int b200icp_s2m_init(const void* scan, int32_t dtype, int32_t n, const double* init_pose,
                      double* src64, double* prev_nn, b200icp_s2m_state* state, void* stream) {
-  if (!scan || !src64 || !state || n < 1) return fail("s2m_init: bad arguments", B200ICP_ERR_INVALID_ARGUMENT);
-  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) return fail("s2m_init: bad dtype", B200ICP_ERR_INVALID_ARGUMENT);
+  if (!scan || !src64 || !state || n < 1) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_init: bad arguments");
+  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_init: bad dtype");
   s2m_init_kernel<<<(n + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       scan, dtype, n, init_pose, src64, prev_nn, state);
-  return cuda_check("s2m_init_kernel");
+  return check_launch("s2m_init_kernel");
 }
 
 int b200icp_s2m_search(const b200icp_s2m_shard* shard, const b200icp_s2m_tables* tables, double* src64,
@@ -1012,18 +983,18 @@ int b200icp_s2m_search(const b200icp_s2m_shard* shard, const b200icp_s2m_tables*
                        void* const* peers, int32_t world, int32_t rank, b200icp_s2m_state* state,
                        void* scratch, void* stream) {
   if (!shard || !tables || !src64 || !state || !scratch || n < 1)
-    return fail("s2m_search: bad arguments", B200ICP_ERR_INVALID_ARGUMENT);
-  if (!records && !peers) return fail("s2m_search: needs records or peers", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_search: bad arguments");
+  if (!records && !peers) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_search: needs records or peers");
   if (peers && (world < 1 || world > kMaxWorld || rank < 0 || rank >= world))
-    return fail("s2m_search: bad world / rank", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_search: bad world / rank");
   if (!tables->chunk_circle || !tables->super_circle || tables->n_chunks_total % kSuper ||
       tables->first_local_chunk % kSuper || tables->n_local_chunks % kSuper ||
       tables->first_local_chunk + tables->n_local_chunks > tables->n_chunks_total ||
       (int64_t)tables->n_local_chunks != b200icp_s2m_padded_chunks(shard->m))
-    return fail("s2m_search: inconsistent circle tables", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_search: inconsistent circle tables");
   SearchArgs a;
   if ((shard->sorted_points == nullptr) != (shard->order == nullptr))
-    return fail("s2m_search: sorted_points and order go together", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_search: sorted_points and order go together");
   a.points = shard->sorted_points ? shard->sorted_points : shard->points; a.order = shard->order;
   a.m = shard->m; a.global_offset = shard->global_offset; a.dtype = shard->dtype;
   a.chunk_circle = tables->chunk_circle; a.super_circle = tables->super_circle;
@@ -1033,7 +1004,7 @@ int b200icp_s2m_search(const b200icp_s2m_shard* shard, const b200icp_s2m_tables*
   a.world = world; a.rank = rank; a.state = state; a.scratch = reinterpret_cast<unsigned*>(scratch);
   s2m_search_kernel<<<(n + kSearchWarps - 1) / kSearchWarps, kSearchWarps * 32, 0,
                       reinterpret_cast<cudaStream_t>(stream)>>>(a);
-  return cuda_check("s2m_search_kernel");
+  return check_launch("s2m_search_kernel");
 }
 
 int b200icp_s2m_update(const b200icp_s2m_record* records_all, void* inbox, int32_t n_ranks, const double* src64,
@@ -1041,29 +1012,29 @@ int b200icp_s2m_update(const b200icp_s2m_record* records_all, void* inbox, int32
                        double max_corr_dist, int32_t* idx_out, b200icp_s2m_state* state, void* scratch,
                        void* stream) {
   if ((!records_all && !inbox) || !src64 || !prev_nn || !state || !scratch || n < 1 || n_ranks < 1 || n_ranks > kMaxWorld)
-    return fail("s2m_update: bad arguments", B200ICP_ERR_INVALID_ARGUMENT);
+    return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_update: bad arguments");
   UpdateArgs a;
   a.records_all = records_all; a.inbox = inbox; a.n_ranks = n_ranks; a.src64 = src64; a.prev_nn = prev_nn;
   a.n = n; a.max_iterations = max_iterations; a.tolerance = tolerance; a.max_corr_dist = max_corr_dist;
   a.idx_out = idx_out; a.state = state; a.scratch = reinterpret_cast<unsigned*>(scratch);
   s2m_update_kernel<<<update_ctas(n), kUpdateThreads, 0, reinterpret_cast<cudaStream_t>(stream)>>>(a);
-  return cuda_check("s2m_update_kernel");
+  return check_launch("s2m_update_kernel");
 }
 
 int b200icp_s2m_finish(double* src64, int32_t n, b200icp_s2m_state* state, void* scratch, void* stream) {
-  if (!src64 || !state || !scratch || n < 1) return fail("s2m_finish: bad arguments", B200ICP_ERR_INVALID_ARGUMENT);
+  if (!src64 || !state || !scratch || n < 1) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_finish: bad arguments");
   s2m_finish_kernel<<<(n + 255) / 256, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       src64, n, state, reinterpret_cast<unsigned*>(scratch));
-  return cuda_check("s2m_finish_kernel");
+  return check_launch("s2m_finish_kernel");
 }
 
 int b200icp_peer_alloc(int64_t bytes, void** ptr_out, void* handle_out) {
-  if (bytes < 1 || !ptr_out || !handle_out) return fail("peer_alloc: bad arguments", B200ICP_ERR_INVALID_ARGUMENT);
+  if (bytes < 1 || !ptr_out || !handle_out) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "peer_alloc: bad arguments");
   void* p = nullptr;
-  if (cudaMalloc(&p, (size_t)bytes) != cudaSuccess) return cuda_check("cudaMalloc");
-  if (cudaMemset(p, 0, (size_t)bytes) != cudaSuccess) return cuda_check("cudaMemset");
+  if (cudaMalloc(&p, (size_t)bytes) != cudaSuccess) return check_launch("cudaMalloc");
+  if (cudaMemset(p, 0, (size_t)bytes) != cudaSuccess) return check_launch("cudaMemset");
   cudaIpcMemHandle_t h;
-  if (cudaIpcGetMemHandle(&h, p) != cudaSuccess) { cudaFree(p); return cuda_check("cudaIpcGetMemHandle"); }
+  if (cudaIpcGetMemHandle(&h, p) != cudaSuccess) { cudaFree(p); return check_launch("cudaIpcGetMemHandle"); }
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
   memcpy(handle_out, &h, 64);
   *ptr_out = p;
@@ -1071,22 +1042,22 @@ int b200icp_peer_alloc(int64_t bytes, void** ptr_out, void* handle_out) {
 }
 
 int b200icp_peer_open(const void* handle, void** ptr_out) {
-  if (!handle || !ptr_out) return fail("peer_open: bad arguments", B200ICP_ERR_INVALID_ARGUMENT);
+  if (!handle || !ptr_out) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "peer_open: bad arguments");
   cudaIpcMemHandle_t h;
   memcpy(&h, handle, 64);
   void* p = nullptr;
-  if (cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) return cuda_check("cudaIpcOpenMemHandle");
+  if (cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) return check_launch("cudaIpcOpenMemHandle");
   *ptr_out = p;
   return B200ICP_OK;
 }
 
 int b200icp_peer_close(void* ptr) {
-  if (ptr && cudaIpcCloseMemHandle(ptr) != cudaSuccess) return cuda_check("cudaIpcCloseMemHandle");
+  if (ptr && cudaIpcCloseMemHandle(ptr) != cudaSuccess) return check_launch("cudaIpcCloseMemHandle");
   return B200ICP_OK;
 }
 
 int b200icp_peer_free(void* ptr) {
-  if (ptr && cudaFree(ptr) != cudaSuccess) return cuda_check("cudaFree");
+  if (ptr && cudaFree(ptr) != cudaSuccess) return check_launch("cudaFree");
   return B200ICP_OK;
 }
 

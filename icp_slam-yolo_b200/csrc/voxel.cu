@@ -20,9 +20,7 @@
 #include <cstdint>
 #include <cstdio>
 
-#include "b200icp.h"
-
-void b200icp_set_error_str(const char* msg);
+#include "common.cuh"
 
 namespace {
 
@@ -117,7 +115,7 @@ __global__ void __launch_bounds__(1024) voxel_scan_kernel(const int32_t* flag, i
   int32_t inc = s;                                      // warp-shuffle scan of the segment sums
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
-    const int32_t v = __shfl_up_sync(0xffffffffu, inc, o);
+    const int32_t v = __shfl_up_sync(kFull, inc, o);
     if (lane >= o) inc += v;
   }
   if (lane == 31) tot[warp] = inc;
@@ -127,7 +125,7 @@ __global__ void __launch_bounds__(1024) voxel_scan_kernel(const int32_t* flag, i
     int32_t winc = w;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-      const int32_t v = __shfl_up_sync(0xffffffffu, winc, o);
+      const int32_t v = __shfl_up_sync(kFull, winc, o);
       if (lane >= o) winc += v;
     }
     tot[lane] = winc - w;
@@ -161,11 +159,6 @@ VoxelWs voxel_layout(int64_t n) {
   return w;
 }
 
-int vfail(const char* msg, int code) {
-  b200icp_set_error_str(msg);
-  return code;
-}
-
 }  // namespace
 
 extern "C" {
@@ -178,11 +171,11 @@ int64_t b200icp_voxel_workspace_bytes(int64_t n) {
 int b200icp_voxel_downsample(const void* points, int32_t dtype, int64_t n, double voxel_size,
                              void* out_points, int64_t* count_out, void* workspace,
                              int64_t workspace_bytes, void* stream) {
-  if (!points || !out_points || !count_out || !workspace) return vfail("voxel_downsample: NULL pointer", B200ICP_ERR_INVALID_ARGUMENT);
-  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) return vfail("voxel_downsample: bad dtype", B200ICP_ERR_INVALID_ARGUMENT);
-  if (n < 1 || n > 0x7fffffffLL || !(voxel_size > 0.0)) return vfail("voxel_downsample: need n >= 1 and voxel_size > 0", B200ICP_ERR_INVALID_ARGUMENT);
+  if (!points || !out_points || !count_out || !workspace) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "voxel_downsample: NULL pointer");
+  if (dtype != B200ICP_F32 && dtype != B200ICP_F64) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "voxel_downsample: bad dtype");
+  if (n < 1 || n > 0x7fffffffLL || !(voxel_size > 0.0)) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "voxel_downsample: need n >= 1 and voxel_size > 0");
   const VoxelWs w = voxel_layout(n);
-  if (workspace_bytes < w.total) return vfail("voxel_downsample: workspace too small", B200ICP_ERR_INVALID_ARGUMENT);
+  if (workspace_bytes < w.total) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "voxel_downsample: workspace too small");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   unsigned char* base = reinterpret_cast<unsigned char*>(workspace);
   uint64_t* keys_in = reinterpret_cast<uint64_t*>(base + w.keys_in);
@@ -199,16 +192,16 @@ int b200icp_voxel_downsample(const void* points, int32_t dtype, int64_t n, doubl
   size_t cub_bytes = w.cub_bytes;
   cudaError_t e = cub::DeviceRadixSort::SortPairs(base + w.cub, cub_bytes, keys_in, keys_out, idx_in, idx_out,
                                                   (int)n, 0, 64, st);
-  if (e != cudaSuccess) return vfail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
+  if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "%s", cudaGetErrorString(e));
   voxel_key_y_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, inv, idx_out, keys_in);
   cub_bytes = w.cub_bytes;
   e = cub::DeviceRadixSort::SortPairs(base + w.cub, cub_bytes, keys_in, keys_out, idx_out, idx_in, (int)n, 0, 64, st);
-  if (e != cudaSuccess) return vfail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
+  if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "%s", cudaGetErrorString(e));
   voxel_head_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, inv, keys_out, idx_in, flags);
   voxel_scan_kernel<<<1, 1024, 0, st>>>(flags, n, rank);
   voxel_emit_kernel<<<blocks, 256, 0, st>>>(points, dtype, n, keys_out, idx_in, flags, rank, out_points, count_out);
   e = cudaGetLastError();
-  if (e != cudaSuccess) return vfail(cudaGetErrorString(e), B200ICP_ERR_CUDA);
+  if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "%s", cudaGetErrorString(e));
   return B200ICP_OK;
 }
 

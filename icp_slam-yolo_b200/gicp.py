@@ -16,8 +16,8 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .registration import (AlignResult, ScanTable, _check_out, _check_pairs, _default_pairs, _problem, _ptr,
-                           _require_cuda, _stream_ptr, alloc_outputs)
+from .registration import (AlignResult, ScanTable, _check_out, _check_pairs, _default_pairs, _init_pose_ptr,
+                           _outputs, _problem, _ptr, _require_cuda, _stream_ptr, alloc_outputs)
 
 
 def estimate_covariances(table: ScanTable, k: int = 20, epsilon: float = 1e-3, stream=None) -> torch.Tensor:
@@ -72,19 +72,10 @@ def gicp_pairs(src: ScanTable, tgt: ScanTable, src_cov: torch.Tensor, tgt_cov: t
     opt.max_iterations = int(max_iterations)
     opt.max_corr_dist = 0.0 if max_corr_dist is None else float(max_corr_dist)
     opt.relative_fitness, opt.relative_rmse = float(relative_fitness), float(relative_rmse)
-    if init_pose is not None:
-        if init_pose.dtype != torch.float64 or tuple(init_pose.shape) != (b, 6):
-            raise ValueError("init_pose must be float64 [n_pairs, 6]")
-        _require_cuda(init_pose, "init_pose")
-        opt.init_pose = init_pose.data_ptr()
-    o = _cabi.Outputs()
-    o.pose_total, o.pose_last = out.pose_total.data_ptr(), _ptr(out.pose_last)
-    o.error, o.rmse = out.error.data_ptr(), _ptr(out.rmse)
-    o.inliers, o.iterations = _ptr(out.inliers), out.iterations.data_ptr()
-    o.indices, o.src_final, o.index_history = _ptr(out.indices), _ptr(out.src_final), _ptr(out.index_history)
+    opt.init_pose = _init_pose_ptr(init_pose, b)
     with torch.cuda.device(dev):
-        rc = _cabi.lib().b200icp_gicp_batch(C.byref(pr), b, C.byref(opt), _ptr(src_cov), _ptr(tgt_cov), C.byref(o),
-                                            _stream_ptr(stream))
+        rc = _cabi.lib().b200icp_gicp_batch(C.byref(pr), b, C.byref(opt), _ptr(src_cov), _ptr(tgt_cov),
+                                            C.byref(_outputs(out)), _stream_ptr(stream))
     _cabi.check(rc, "b200icp_gicp_batch")
     return out
 

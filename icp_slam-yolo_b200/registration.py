@@ -16,6 +16,9 @@ import torch
 from . import _cabi
 
 _DTYPES = {torch.float32: _cabi.F32, torch.float64: _cabi.F64}
+# kernel="auto" takes the CTA-per-pair kernel up to this many pairs, the W-warps-per-pair kernel above
+# (kAutoCtaPairs in csrc/b200icp.cu)
+_AUTO_CTA_PAIRS = 512
 _PAIRINGS = {"rowwise": _cabi.PAIR_ROWWISE, "explicit": _cabi.PAIR_EXPLICIT,
              "triangle": _cabi.PAIR_TRIANGLE}
 
@@ -206,6 +209,33 @@ def _check_out(out: "AlignResult", b: int, src_pitch: int, max_iterations: int, 
                              f"(the kernel strides it by max_iterations), got {tuple(h.shape)}")
 
 
+def _kernel_flags(kernel: str, dense_sweep: bool, sweep_reuse: bool = True, pair_warps: int = 0) -> int:
+    """b200icp_options.flags / the flags of b200icp_nn_batch for the Python-side kernel choice."""
+    return ((_cabi.FLAG_DENSE_SWEEP if dense_sweep else 0) | (0 if sweep_reuse else _cabi.FLAG_NO_SWEEP_REUSE) |
+            {"auto": 0, "warp": _cabi.FLAG_WARP_KERNEL, "cta": _cabi.FLAG_CTA_KERNEL}[kernel] |
+            ((int(pair_warps) & 7) << _cabi.FLAG_PAIR_WARPS_SHIFT))
+
+
+def _init_pose_ptr(init_pose: Optional[torch.Tensor], b: int):
+    """Device pointer of an optional float64 [b, 6] initial pose (None: identity)."""
+    if init_pose is None:
+        return None
+    if init_pose.dtype != torch.float64 or tuple(init_pose.shape) != (b, 6):
+        raise ValueError("init_pose must be float64 [n_pairs, 6]")
+    _require_cuda(init_pose, "init_pose")
+    return init_pose.data_ptr()
+
+
+def _outputs(out: "AlignResult") -> "_cabi.Outputs":
+    """The b200icp_outputs view of a result buffer; pose_total, error and iterations are required."""
+    o = _cabi.Outputs()
+    o.pose_total, o.error, o.iterations = out.pose_total.data_ptr(), out.error.data_ptr(), out.iterations.data_ptr()
+    o.pose_last, o.rmse, o.inliers = _ptr(out.pose_last), _ptr(out.rmse), _ptr(out.inliers)
+    o.indices, o.src_final, o.index_history = _ptr(out.indices), _ptr(out.src_final), _ptr(out.index_history)
+    o.evaluated_pairs = _ptr(out.evaluated_pairs)
+    return o
+
+
 def nn_search(src: ScanTable, tgt: ScanTable, *, n_pairs: Optional[int] = None,
               pairing: str = "rowwise", src_row=None, tgt_row=None, first_pair: int = 0,
               want_dist2: bool = True, out_idx=None, out_dist2=None, validate_rows: bool = False,
@@ -229,9 +259,8 @@ def nn_search(src: ScanTable, tgt: ScanTable, *, n_pairs: Optional[int] = None,
     if d2 is None and want_dist2:
         d2 = torch.empty((b, src.pitch), dtype=torch.float64, device=dev)
     with torch.cuda.device(dev):
-        flags = ((_cabi.FLAG_DENSE_SWEEP if dense_sweep else 0) |
-                 {"auto": 0, "warp": _cabi.FLAG_WARP_KERNEL, "cta": _cabi.FLAG_CTA_KERNEL}[kernel])
-        rc = _cabi.lib().b200icp_nn_batch(C.byref(pr), b, _ptr(idx), _ptr(d2), flags, _stream_ptr(stream))
+        rc = _cabi.lib().b200icp_nn_batch(C.byref(pr), b, _ptr(idx), _ptr(d2), _kernel_flags(kernel, dense_sweep),
+                                          _stream_ptr(stream))
     _cabi.check(rc, "b200icp_nn_batch")
     return idx, d2
 
@@ -289,24 +318,11 @@ def align_pairs(src: ScanTable, tgt: ScanTable, *, n_pairs: Optional[int] = None
                             want_stats=want_stats)
     opt = _cabi.Options()
     opt.max_iterations = int(max_iterations)
-    opt.flags = ((_cabi.FLAG_DENSE_SWEEP if dense_sweep else 0) | (0 if sweep_reuse else _cabi.FLAG_NO_SWEEP_REUSE) |
-                 {"auto": 0, "warp": _cabi.FLAG_WARP_KERNEL, "cta": _cabi.FLAG_CTA_KERNEL}[kernel] |
-                 ((int(pair_warps) & 7) << _cabi.FLAG_PAIR_WARPS_SHIFT))
+    opt.flags = _kernel_flags(kernel, dense_sweep, sweep_reuse, pair_warps)
     opt.tolerance = float(tolerance)
     opt.max_corr_dist = 0.0 if max_corr_dist is None else float(max_corr_dist)
-    if init_pose is not None:
-        if init_pose.dtype != torch.float64 or tuple(init_pose.shape) != (b, 6):
-            raise ValueError("init_pose must be float64 [n_pairs, 6]")
-        _require_cuda(init_pose, "init_pose")
-        opt.init_pose = init_pose.data_ptr()
-    o = _cabi.Outputs()
-    o.pose_total, o.pose_last = out.pose_total.data_ptr(), out.pose_last.data_ptr()
-    o.error, o.rmse = out.error.data_ptr(), out.rmse.data_ptr()
-    o.inliers, o.iterations = out.inliers.data_ptr(), out.iterations.data_ptr()
-    o.indices = None if out.indices is None else out.indices.data_ptr()
-    o.src_final = None if out.src_final is None else out.src_final.data_ptr()
-    o.index_history = None if out.index_history is None else out.index_history.data_ptr()
-    o.evaluated_pairs = None if out.evaluated_pairs is None else out.evaluated_pairs.data_ptr()
+    opt.init_pose = _init_pose_ptr(init_pose, b)
+    o = _outputs(out)
     with torch.cuda.device(dev):
         rc = _cabi.lib().b200icp_align_batch(C.byref(pr), b, C.byref(opt), C.byref(o),
                                              _stream_ptr(stream))
@@ -421,7 +437,7 @@ class HostPipeline:
         self.compute_streams = [torch.cuda.Stream(device=self.device) for _ in range(self.nbuf)]
         # one fused kernel for every chunk, chosen on the size of the whole batch: results must not
         # depend on how the batch is cut (the two kernels agree to ~1e-12, not bit for bit)
-        self.kernel = "warp" if self.n_pairs > 512 else "cta"
+        self.kernel = "warp" if self.n_pairs > _AUTO_CTA_PAIRS else "cta"
         pin = lambda *shape, dt: torch.empty(shape, dtype=dt, pin_memory=True)
         from . import hostmem
         with hostmem.near_gpu(self.device.index if self.device.index is not None else torch.cuda.current_device()):

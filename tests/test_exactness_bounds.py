@@ -2,7 +2,7 @@
 
 They restate, in NumPy float32 / float64 arithmetic, (a) the skip test of the scan-to-map FP32 filter
 (`Fp32Filter`, `filter_threshold`, `scan_round` in csrc/scan2map.cu) and (b) the bounds of the 16-target
-decision of the pair kernel (`in_group_decide` in csrc/b200icp.cu: low mantissa byte replaced by the
+decision of the pair kernel (`in_group_decide` in csrc/align_pair.cu: low mantissa byte replaced by the
 slot number), and check on adversarial inputs the properties the kernels' proofs use:
   (a) a skipped point is farther than the best so far in the EXACT float64 arithmetic of `consider`;
   (b) `ubd` >= the exact distance to the winner, `los` <= the exact distance to every other target, and
