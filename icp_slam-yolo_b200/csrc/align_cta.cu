@@ -4,7 +4,7 @@
 // Reference behaviour being replaced (paths relative to the reference repo):
 //   labels_segmentation/icp.py:28-53  icp()                 -> icp_align_kernel
 //   labels_segmentation/icp.py:37-38  KDTree(B).query(src)   -> nn_candidates + nn_resolve
-//   labels_segmentation/icp.py:5-26   best_fit_transform()   -> pose solve inside icp_align_kernel
+//   labels_segmentation/icp.py:5-26   best_fit_transform()   -> kabsch_increment (icp_step.cuh) in icp_align_kernel
 //
 // Kernel design (see DESIGN.md):
 //   * one CTA per scan pair, the whole <=max_iterations loop on the device;
@@ -19,7 +19,8 @@
 //     source in float64 and a shuffle argmin with (distance, index) ordering decides;
 //   * all O(N) state (source points, centroid / covariance sums, pose, error) is float64,
 //     reduced by warp shuffles + one shared-memory hop, every thread solving the 2x2
-//     Kabsch problem in closed form redundantly (no broadcast step).
+//     Kabsch problem in closed form redundantly (no broadcast step); the update step itself
+//     (sums, Kabsch, apply, compose, outputs) is icp_step.cuh's.
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -52,16 +53,13 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) nn_pair_ke
 
   int64_t srow, trow;
   resolve_rows(pr, p, srow, trow);
-  const int n = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
-  const int m = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+  int n, m;
+  row_lengths(pr, srow, trow, n, m);
   int32_t* idx_out = a.nn_idx + p * pr.src_pitch;
   double* d2_out = a.nn_dist2 ? a.nn_dist2 + p * pr.src_pitch : nullptr;
 
   if (n <= 0 || m <= 0) {
-    for (int i = tid; i < pr.src_pitch; i += nthreads) {
-      idx_out[i] = -1;
-      if (d2_out) d2_out[i] = CUDART_INF;
-    }
+    nn_fill_none(idx_out, d2_out, tid, pr.src_pitch, nthreads);
     return;
   }
   stage_targets(pr.tgt_points, pr.dtype, trow * pr.tgt_pitch, m, t, tid, nthreads, warp,
@@ -108,16 +106,12 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) icp_align_
 
   int64_t srow, trow;
   resolve_rows(pr, p, srow, trow);
-  const int n = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
-  const int m = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+  int n, m;
+  row_lengths(pr, srow, trow, n, m);
 
   // cumulative pose (src = Rt * A + tt) starts at the initial pose (gicp_lidar.py:32 shape)
-  double R00 = 1.0, R01 = 0.0, R10 = 0.0, R11 = 1.0, T0 = 0.0, T1 = 0.0;
-  if (op.init_pose) {
-    const double* ip = op.init_pose + p * 6;
-    R00 = ip[0]; R01 = ip[1]; R10 = ip[2]; R11 = ip[3]; T0 = ip[4]; T1 = ip[5];
-  }
-  double c_last = 1.0, s_last = 0.0, t0_last = 0.0, t1_last = 0.0;   // last increment
+  Se2 pose = load_init_pose(op.init_pose, p);
+  Increment last{1.0, 0.0, 0.0, 0.0};
   double err = CUDART_INF, mean_d2 = CUDART_INF;
   int iters = 0, inl = 0;
 
@@ -136,13 +130,9 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) icp_align_
       const int i = tid + k * nthreads;
       valid[k] = i < n;
       if (valid[k]) {
-        const double2 q = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i);
-        if (op.init_pose) {
-          sx[k] = R00 * q.x + R01 * q.y + T0;
-          sy[k] = R10 * q.x + R11 * q.y + T1;
-        } else {
-          sx[k] = q.x; sy[k] = q.y;          // icp.py:32  src = copy(A)
-        }
+        double2 q = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i);   // icp.py:32  src = copy(A)
+        if (op.init_pose) q = apply(pose, q);
+        sx[k] = q.x; sy[k] = q.y;
       }
     }
     const double gate = op.max_corr_dist;
@@ -165,11 +155,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) icp_align_
           const double dist = sqrt(d2[k]);
           if (!use_gate || dist < gate) {
             const double2 b = t.t64[idx[k]];
-            const double ax = sx[k] - t.ox, ay = sy[k] - t.oy;
-            const double qx = b.x - t.ox, qy = b.y - t.oy;
-            r[0] += ax; r[1] += ay; r[2] += qx; r[3] += qy;
-            r[4] = fma(ax, qx, r[4]); r[5] = fma(ax, qy, r[5]);
-            r[6] = fma(ay, qx, r[6]); r[7] = fma(ay, qy, r[7]);
+            add_match(r, sx[k] - t.ox, sy[k] - t.oy, b.x - t.ox, b.y - t.oy);
             r[8] += dist; r[9] += d2[k]; r[10] += 1.0;
           }
         }
@@ -189,38 +175,18 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) icp_align_
         }
       }
       const double inv = use_gate ? 1.0 / cnt : inv_n;
-      const double max_ = r[0] * inv, may_ = r[1] * inv;        // centroids rel. origin (icp.py:10-11)
-      const double mbx = r[2] * inv, mby = r[3] * inv;
       const double mean_error = r[8] * inv;                     // icp.py:48
-      // ---- closed-form 2D Kabsch: the proper rotation the SVD route (icp.py:17-23) returns
-      const double h00 = fma(-r[0], mbx, r[4]), h01 = fma(-r[0], mby, r[5]);
-      const double h10 = fma(-r[1], mbx, r[6]), h11 = fma(-r[1], mby, r[7]);
-      const double num = h01 - h10, den = h00 + h11;
-      const double h2 = fma(num, num, den * den);
-      double cs = 1.0, sn = 0.0;
-      if (h2 > 0.0) {
-        const double rh = rsqrt(h2);
-        cs = den * rh; sn = num * rh;
-      }
-      const double cax = t.ox + max_, cay = t.oy + may_;
-      const double tx = (t.ox + mbx) - (cs * cax - sn * cay);   // icp.py:25
-      const double ty = (t.oy + mby) - (sn * cax + cs * cay);
+      const Increment d = kabsch_increment(r, inv, t.ox, t.oy, t.ox, t.oy);
       // ---- apply (icp.py:45) and compose the cumulative pose
 #pragma unroll
       for (int k = 0; k < S; ++k) {
         if (valid[k]) {
-          const double x = sx[k], y = sy[k];
-          sx[k] = cs * x - sn * y + tx;
-          sy[k] = sn * x + cs * y + ty;
+          const double2 v = apply(d, make_double2(sx[k], sy[k]));
+          sx[k] = v.x; sy[k] = v.y;
         }
       }
-      {
-        const double n00 = cs * R00 - sn * R10, n01 = cs * R01 - sn * R11;
-        const double n10 = sn * R00 + cs * R10, n11 = sn * R01 + cs * R11;
-        const double nt0 = cs * T0 - sn * T1 + tx, nt1 = sn * T0 + cs * T1 + ty;
-        R00 = n00; R01 = n01; R10 = n10; R11 = n11; T0 = nt0; T1 = nt1;
-      }
-      c_last = cs; s_last = sn; t0_last = tx; t1_last = ty;
+      pose = compose(d, pose);
+      last = d;
       err = mean_error; mean_d2 = r[9] * inv; inl = (int)(cnt + 0.5);
       iters = it + 1;
       // ---- convergence (icp.py:49-51); identical in every thread
@@ -229,19 +195,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) icp_align_
     }
   }
 
-  if (tid == 0) {
-    double* pt = out.pose_total + p * 6;
-    pt[0] = R00; pt[1] = R01; pt[2] = R10; pt[3] = R11; pt[4] = T0; pt[5] = T1;
-    if (out.pose_last) {
-      double* pl = out.pose_last + p * 6;
-      pl[0] = c_last; pl[1] = -s_last; pl[2] = s_last; pl[3] = c_last;
-      pl[4] = t0_last; pl[5] = t1_last;
-    }
-    out.error[p] = err;
-    if (out.rmse) out.rmse[p] = sqrt(mean_d2);
-    if (out.inliers) out.inliers[p] = inl;
-    out.iterations[p] = iters;
-  }
+  if (tid == 0) write_pair_result(out, p, pose, last, err, mean_d2, inl, iters);
   if (out.indices || out.src_final) {
 #pragma unroll
     for (int k = 0; k < S; ++k) {
@@ -254,8 +208,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, B200ICP_MIN_BLOCKS) icp_align_
             if (ran) {
               v = make_double2(sx[k], sy[k]);
             } else {     // nothing ran: report the (pre-transformed) input
-              const double2 q = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i);
-              v = make_double2(R00 * q.x + R01 * q.y + T0, R10 * q.x + R11 * q.y + T1);
+              v = apply(pose, load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i));
             }
           }
           reinterpret_cast<double2*>(out.src_final)[p * pr.src_pitch + i] = v;

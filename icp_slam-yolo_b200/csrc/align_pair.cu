@@ -1,6 +1,7 @@
 // align_pair.cu -- the throughput kernels: the fused ICP loop with W warps per pair sharing one
 // target tile (icp_align_pair_kernel), and the one-warp-per-pair nearest-neighbour search
-// (nn_warp_kernel) built from its search phase.  DESIGN.md has the measurements.
+// (nn_warp_kernel) built from its search phase.  DESIGN.md has the measurements.  The update step
+// (sums, Kabsch, apply, compose, outputs) is icp_step.cuh's.
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -84,39 +85,6 @@ __device__ __forceinline__ float key_eps(float cs, float tmax, unsigned keep) {
   return rel * 2.02f * s * s;
 }
 
-// Candidate sweep over the warp tile (expanded form, packed FFMA2), every group.
-template <int S>
-__device__ __forceinline__ void warp_candidates(const PairTile& t, const float (&sx)[S],
-                                                const float (&sy)[S], Cand3<S>& c, unsigned keep) {
-  const float4* __restrict__ g4 = reinterpret_cast<const float4*>(t.tile);
-  float a[S], b[S];
-#pragma unroll
-  for (int k = 0; k < S; ++k) {
-    float vx = -2.0f * sx[k], vy = -2.0f * sy[k];
-    asm volatile("" : "+f"(vx), "+f"(vy));
-    a[k] = vx; b[k] = vy;
-    c.kb[k] = CUDART_INF_F; c.ks[k] = CUDART_INF_F; c.kt[k] = CUDART_INF_F;
-  }
-  const int ngroups = t.ngroups;
-#pragma unroll 1
-  for (int g = 0; g < ngroups; ++g) {
-    const float4 xa = g4[6 * g], xb = g4[6 * g + 1];
-    const float4 ya = g4[6 * g + 2], yb = g4[6 * g + 3];
-    const float4 qa = g4[6 * g + 4], qb = g4[6 * g + 5];
-#pragma unroll
-    for (int k = 0; k < S; ++k) {
-      const float2 ak = make_float2(a[k], a[k]), bk = make_float2(b[k], b[k]);
-      const float2 e01 = __ffma2_rn(ak, make_float2(xa.x, xa.y), __ffma2_rn(bk, make_float2(ya.x, ya.y), make_float2(qa.x, qa.y)));
-      const float2 e23 = __ffma2_rn(ak, make_float2(xa.z, xa.w), __ffma2_rn(bk, make_float2(ya.z, ya.w), make_float2(qa.z, qa.w)));
-      const float2 e45 = __ffma2_rn(ak, make_float2(xb.x, xb.y), __ffma2_rn(bk, make_float2(yb.x, yb.y), make_float2(qb.x, qb.y)));
-      const float2 e67 = __ffma2_rn(ak, make_float2(xb.z, xb.w), __ffma2_rn(bk, make_float2(yb.z, yb.w), make_float2(qb.z, qb.w)));
-      const float m = fminf(fminf(fminf(e01.x, e01.y), fminf(e23.x, e23.y)),
-                            fminf(fminf(e45.x, e45.y), fminf(e67.x, e67.y)));
-      track3<S>(c, k, m, (unsigned)g, keep);
-    }
-  }
-}
-
 // One group of 8 targets against the S sources of a lane (expanded form, packed FFMA2),
 // split into the shared-memory loads and the arithmetic so the candidate loop can fetch the
 // next group while the current one is being evaluated.
@@ -147,6 +115,23 @@ __device__ __forceinline__ void eval_group(const GroupRegs& r, int g, const floa
                           fminf(fminf(e45.x, e45.y), fminf(e67.x, e67.y)));
     track3<S>(c, k, m, (unsigned)g, keep);
   }
+}
+
+// Candidate sweep over the warp tile (expanded form, packed FFMA2), every group.
+template <int S>
+__device__ __forceinline__ void warp_candidates(const PairTile& t, const float (&sx)[S],
+                                                const float (&sy)[S], Cand3<S>& c, unsigned keep) {
+  float a[S], b[S];
+#pragma unroll
+  for (int k = 0; k < S; ++k) {
+    float vx = -2.0f * sx[k], vy = -2.0f * sy[k];
+    asm volatile("" : "+f"(vx), "+f"(vy));
+    a[k] = vx; b[k] = vy;
+    c.kb[k] = CUDART_INF_F; c.ks[k] = CUDART_INF_F; c.kt[k] = CUDART_INF_F;
+  }
+  const int ngroups = t.ngroups;
+#pragma unroll 1
+  for (int g = 0; g < ngroups; ++g) eval_group<S>(load_group(t, g), g, a, b, c, keep);
 }
 
 // Evaluate every group whose bit is set in `mask` (groups base_g + bit).
@@ -333,8 +318,8 @@ __device__ __forceinline__ int fold10_owner(int lane) {
 }
 
 struct PairCtx {            // shared memory; touched by thread 0 only until the final barrier
-  double R[4], T[2];        // cumulative pose, src = R A + T
-  double last[4];           // last increment: cos, sin, tx, ty
+  Se2 pose;                 // cumulative pose, src = R A + T
+  Increment last;           // last increment
   double err, mean_d2;
   int iters, inl;
   unsigned long long evals; // pair evaluations executed by the sweeps of all warps
@@ -660,8 +645,8 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
 
   int64_t srow, trow;
   resolve_rows(pr, p, srow, trow);
-  const int n = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
-  const int m = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+  int n, m;
+  row_lengths(pr, srow, trow, n, m);
 
   PairTile t;
   PairCtx* ctx;
@@ -671,14 +656,8 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
 
   const bool ran = n > 0 && m > 0 && op.max_iterations > 0;
   if (tid == 0) {
-    double R00 = 1.0, R01 = 0.0, R10 = 0.0, R11 = 1.0, T0 = 0.0, T1 = 0.0;
-    if (op.init_pose) {
-      const double* ip = op.init_pose + p * 6;
-      R00 = ip[0]; R01 = ip[1]; R10 = ip[2]; R11 = ip[3]; T0 = ip[4]; T1 = ip[5];
-    }
-    ctx->R[0] = R00; ctx->R[1] = R01; ctx->R[2] = R10; ctx->R[3] = R11;
-    ctx->T[0] = T0; ctx->T[1] = T1;
-    ctx->last[0] = 1.0; ctx->last[1] = 0.0; ctx->last[2] = 0.0; ctx->last[3] = 0.0;
+    ctx->pose = load_init_pose(op.init_pose, p);
+    ctx->last = Increment{1.0, 0.0, 0.0, 0.0};
     ctx->err = CUDART_INF; ctx->mean_d2 = CUDART_INF;
     ctx->iters = 0; ctx->inl = 0; ctx->evals = 0ull;
   }
@@ -694,10 +673,7 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
       double2 v = make_double2(t.ox, t.oy);                // padding slots: benign, never used
       if (i < n) {
         const double2 q = load_point(pr.src_points, t.dtype, srow * pr.src_pitch + i);
-        v = q;                                             // icp.py:32  src = copy(A)
-        if (op.init_pose)
-          v = make_double2(ctx->R[0] * q.x + ctx->R[1] * q.y + ctx->T[0],
-                           ctx->R[2] * q.x + ctx->R[3] * q.y + ctx->T[1]);
+        v = op.init_pose ? apply(ctx->pose, q) : q;       // icp.py:32  src = copy(A)
         smax = fmaxf(smax, fmaxf(__double2float_ru(fabs(v.x - t.ox)), __double2float_ru(fabs(v.y - t.oy))));
       }
       t.src[i] = v;
@@ -775,11 +751,7 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
               const double2 b = bm[u];
               const double d2 = dist2_f64(s.x, s.y, b);
               const double dist = sqrt_f64_fast(d2);
-              const double ax = s.x - t.ox, ay = s.y - t.oy;
-              const double qx = b.x - t.ox, qy = b.y - t.oy;
-              r[0] += ax; r[1] += ay; r[2] += qx; r[3] += qy;
-              r[4] = fma(ax, qx, r[4]); r[5] = fma(ax, qy, r[5]);
-              r[6] = fma(ay, qx, r[6]); r[7] = fma(ay, qy, r[7]);
+              add_match(r, s.x - t.ox, s.y - t.oy, b.x - t.ox, b.y - t.oy);
               r[8] += dist; r[9] += d2;
             }
             continue;
@@ -801,11 +773,7 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
               const double d2 = dist2_f64(s.x, s.y, b);
               const double dist = sqrt_f64_fast(d2);
               if (!use_gate || dist < op.max_corr_dist) {
-                const double ax = s.x - t.ox, ay = s.y - t.oy;
-                const double qx = b.x - t.ox, qy = b.y - t.oy;
-                r[0] += ax; r[1] += ay; r[2] += qx; r[3] += qy;
-                r[4] = fma(ax, qx, r[4]); r[5] = fma(ax, qy, r[5]);
-                r[6] = fma(ay, qx, r[6]); r[7] = fma(ay, qy, r[7]);
+                add_match(r, s.x - t.ox, s.y - t.oy, b.x - t.ox, b.y - t.oy);
                 r[8] += dist; r[9] += d2;
                 if (!LEAN) r[10] += 1.0;
               }
@@ -847,30 +815,13 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
         break;
       }
       const double inv = use_gate ? 1.0 / cnt : inv_n;
-      const double max_ = r[0] * inv, may_ = r[1] * inv;       // centroids rel. origin (icp.py:10-11)
-      const double mbx = r[2] * inv, mby = r[3] * inv;
       const double mean_error = r[8] * inv;                    // icp.py:48
-      // closed-form 2D Kabsch: the proper rotation the SVD route (icp.py:17-23) returns
-      const double h00 = fma(-r[0], mbx, r[4]), h01 = fma(-r[0], mby, r[5]);
-      const double h10 = fma(-r[1], mbx, r[6]), h11 = fma(-r[1], mby, r[7]);
-      const double num = h01 - h10, den = h00 + h11;
-      const double h2 = fma(num, num, den * den);
-      double cs = 1.0, sn = 0.0;
-      if (h2 > 0.0) {
-        const double rh = rsqrt(h2);
-        cs = den * rh; sn = num * rh;
-      }
-      const double cax = t.ox + max_, cay = t.oy + may_;
-      const double tx = (t.ox + mbx) - (cs * cax - sn * cay);  // icp.py:25
-      const double ty = (t.oy + mby) - (sn * cax + cs * cay);
+      const Increment d = kabsch_increment(r, inv, t.ox, t.oy, t.ox, t.oy);
       for (int base = warp * 64; base < n; base += W * 64) {   // apply (icp.py:45), the blocks this warp summed
 #pragma unroll
         for (int k = 0; k < 2; ++k) {
           const int i = base + k * 32 + lane;
-          if (i < n) {
-            const double2 s = t.src[i];
-            t.src[i] = make_double2(cs * s.x - sn * s.y + tx, sn * s.x + cs * s.y + ty);
-          }
+          if (i < n) t.src[i] = apply(d, t.src[i]);
         }
       }
       if (SC != 2 && W > 1) __syncthreads();               // the next search reads points another warp moved
@@ -882,11 +833,11 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
       // the update itself (a few float64 ulp of the coordinates).  Identical in every thread.
       float mv = 0.f;
       if (a.reuse) {
-        const double c1 = cs - 1.0;
-        const float c1f = (float)c1, snf = (float)sn;
-        const float ddx = (float)(fma(c1, t.ox, -sn * t.oy) + tx), ddy = (float)(fma(sn, t.ox, c1 * t.oy) + ty);
+        const double c1 = d.cs - 1.0;
+        const float c1f = (float)c1, snf = (float)d.sn;
+        const float ddx = (float)(fma(c1, t.ox, -d.sn * t.oy) + d.tx), ddy = (float)(fma(d.sn, t.ox, c1 * t.oy) + d.ty);
         const float rho = sqrtf(fmaf(c1f, c1f, snf * snf)), dd = sqrtf(fmaf(ddx, ddx, ddy * ddy));
-        const float ulp = 1.0e-15f * (fabsf((float)t.ox) + fabsf((float)t.oy) + smax + fabsf((float)tx) + fabsf((float)ty));
+        const float ulp = 1.0e-15f * (fabsf((float)t.ox) + fabsf((float)t.oy) + smax + fabsf((float)d.tx) + fabsf((float)d.ty));
         mv = fmaf(rho, smax, dd) * 1.00001f + ulp + 1e-30f;
         smax = __fadd_ru(smax, mv);
         mv_prev = mv;
@@ -895,12 +846,8 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
       const bool converged = fabs(prev_error - mean_error) < op.tolerance;   // icp.py:49-50
       prev_error = mean_error;                                               // icp.py:51
       if (tid == 0) {            // compose the cumulative pose, record the increment
-        const double R00 = ctx->R[0], R01 = ctx->R[1], R10 = ctx->R[2], R11 = ctx->R[3];
-        const double T0 = ctx->T[0], T1 = ctx->T[1];
-        ctx->R[0] = cs * R00 - sn * R10; ctx->R[1] = cs * R01 - sn * R11;
-        ctx->R[2] = sn * R00 + cs * R10; ctx->R[3] = sn * R01 + cs * R11;
-        ctx->T[0] = cs * T0 - sn * T1 + tx; ctx->T[1] = sn * T0 + cs * T1 + ty;
-        ctx->last[0] = cs; ctx->last[1] = sn; ctx->last[2] = tx; ctx->last[3] = ty;
+        ctx->pose = compose(d, ctx->pose);
+        ctx->last = d;
         ctx->err = mean_error; ctx->mean_d2 = r[9] * inv; ctx->inl = (int)(cnt + 0.5);
         ctx->iters = it + 1;
       }
@@ -913,18 +860,7 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
   if (W > 1) __syncthreads(); else __syncwarp();
   const int iters = ctx->iters;
   if (tid == 0) {
-    double* pt = out.pose_total + p * 6;
-    pt[0] = ctx->R[0]; pt[1] = ctx->R[1]; pt[2] = ctx->R[2]; pt[3] = ctx->R[3];
-    pt[4] = ctx->T[0]; pt[5] = ctx->T[1];
-    if (out.pose_last) {
-      double* pl = out.pose_last + p * 6;
-      pl[0] = ctx->last[0]; pl[1] = -ctx->last[1]; pl[2] = ctx->last[1]; pl[3] = ctx->last[0];
-      pl[4] = ctx->last[2]; pl[5] = ctx->last[3];
-    }
-    out.error[p] = ctx->err;
-    if (out.rmse) out.rmse[p] = sqrt(ctx->mean_d2);
-    if (out.inliers) out.inliers[p] = ctx->inl;
-    out.iterations[p] = iters;
+    write_pair_result(out, p, ctx->pose, ctx->last, ctx->err, ctx->mean_d2, ctx->inl, iters);
     if (out.evaluated_pairs) out.evaluated_pairs[p] = (int64_t)ctx->evals;
   }
   if (idx_out) {
@@ -939,9 +875,7 @@ icp_align_pair_kernel(const KernelArgs a) {      // (the dense sweep holds 6 sou
         if (ran) {
           v = t.src[i];
         } else {         // nothing ran: report the (pre-transformed) input
-          const double2 q = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i);
-          v = make_double2(ctx->R[0] * q.x + ctx->R[1] * q.y + ctx->T[0],
-                           ctx->R[2] * q.x + ctx->R[3] * q.y + ctx->T[1]);
+          v = apply(ctx->pose, load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i));
         }
       }
       dst[i] = v;
@@ -961,15 +895,12 @@ __global__ void __launch_bounds__(32, B200ICP_PAIR_RESIDENT_WARPS) nn_warp_kerne
   const b200icp_problem& pr = a.prob;
   int64_t srow, trow;
   resolve_rows(pr, p, srow, trow);
-  const int n = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
-  const int m = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+  int n, m;
+  row_lengths(pr, srow, trow, n, m);
   int32_t* idx_out = a.nn_idx + p * pr.src_pitch;
   double* d2_out = a.nn_dist2 ? a.nn_dist2 + p * pr.src_pitch : nullptr;
   if (n <= 0 || m <= 0) {
-    for (int i = lane; i < pr.src_pitch; i += 32) {
-      idx_out[i] = -1;
-      if (d2_out) d2_out[i] = CUDART_INF;
-    }
+    nn_fill_none(idx_out, d2_out, lane, pr.src_pitch, 32);
     return;
   }
   PairTile t;
@@ -998,10 +929,7 @@ __global__ void __launch_bounds__(32, B200ICP_PAIR_RESIDENT_WARPS) nn_warp_kerne
       }
     }
   }
-  for (int i = n + lane; i < pr.src_pitch; i += 32) {
-    idx_out[i] = -1;
-    if (d2_out) d2_out[i] = CUDART_INF;
-  }
+  nn_fill_none(idx_out, d2_out, n + lane, pr.src_pitch, 32);
 }
 
 // W-warps-per-pair fused kernel: passes of 64 sources (pruned sweep) or 192 sources (dense sweep),

@@ -1,13 +1,15 @@
 // common.cuh -- what every CUDA source of the library shares: the point layout, the pair
-// addressing of b200icp_problem, the float64 distance every exact decision uses, and the error API
-// behind b200icp_last_error().
+// addressing of b200icp_problem, the float64 distance every exact decision uses, the error API
+// behind b200icp_last_error(), and (icp_step.cuh) the update step of the ICP loop.
 #pragma once
 
 #include <cuda_runtime.h>
+#include <math_constants.h>
 
 #include <cstdint>
 
 #include "b200icp.h"
+#include "icp_step.cuh"
 
 constexpr unsigned kFull = 0xffffffffu;   // all lanes of a warp
 constexpr int kGroup = 8;          // targets per search group
@@ -59,6 +61,20 @@ __device__ __forceinline__ void resolve_rows(const b200icp_problem& pr, int64_t 
     while (i < rows - 2 && tri_offset(i + 1, rows) <= q) ++i;
     trow = i;
     srow = q - tri_offset(i, rows) + i + 1;
+  }
+}
+
+// Valid points of the two rows of a pair: the row length, capped at the pitch.
+__device__ __forceinline__ void row_lengths(const b200icp_problem& pr, int64_t srow, int64_t trow, int& n, int& m) {
+  n = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
+  m = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+}
+
+// "No neighbour" (index -1, d^2 = +inf) in the slots i0, i0 + stride, ... below pitch of an NN row.
+__device__ __forceinline__ void nn_fill_none(int32_t* idx, double* d2, int i0, int pitch, int stride) {
+  for (int i = i0; i < pitch; i += stride) {
+    idx[i] = -1;
+    if (d2) d2[i] = CUDART_INF;
   }
 }
 

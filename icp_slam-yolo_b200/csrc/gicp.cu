@@ -40,10 +40,9 @@ struct GicpArgs {
 
 // R p + t, rounded as the oracle rounds it (no contraction), so that the pivot and a source point at
 // the centroid stay bit-identical.
-__device__ __forceinline__ double2 apply_pose(double r00, double r01, double r10, double r11, double t0,
-                                              double t1, double x, double y) {
-  return make_double2(__dadd_rn(__dadd_rn(__dmul_rn(r00, x), __dmul_rn(r01, y)), t0),
-                      __dadd_rn(__dadd_rn(__dmul_rn(r10, x), __dmul_rn(r11, y)), t1));
+__device__ __forceinline__ double2 apply_pose(const Se2& a, double x, double y) {
+  return make_double2(__dadd_rn(__dadd_rn(__dmul_rn(a.r00, x), __dmul_rn(a.r01, y)), a.tx),
+                      __dadd_rn(__dadd_rn(__dmul_rn(a.r10, x), __dmul_rn(a.r11, y)), a.ty));
 }
 
 template <int S>
@@ -63,17 +62,13 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
 
   int64_t srow, trow;
   resolve_rows(pr, p, srow, trow);
-  const int n = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
-  const int m = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+  int n, m;
+  row_lengths(pr, srow, trow, n, m);
   const int64_t soff = srow * pr.src_pitch, toff = trow * pr.tgt_pitch;
 
-  double R00 = 1.0, R01 = 0.0, R10 = 0.0, R11 = 1.0, T0 = 0.0, T1 = 0.0;
-  if (op.init_pose) {
-    const double* ip = op.init_pose + p * 6;
-    R00 = ip[0]; R01 = ip[1]; R10 = ip[2]; R11 = ip[3]; T0 = ip[4]; T1 = ip[5];
-  }
-  double c_last = 1.0, s_last = 0.0, t0_last = 0.0, t1_last = 0.0;   // last increment
-  double err = CUDART_INF, rmse = CUDART_INF;
+  Se2 P = load_init_pose(op.init_pose, p);
+  Increment last{1.0, 0.0, 0.0, 0.0};
+  double err = CUDART_INF, mean_d2 = CUDART_INF;
   int iters = 0, inl = 0;
 
   double sx[S], sy[S], ca[S][3];
@@ -105,7 +100,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
 #pragma unroll
     for (int k = 0; k < S; ++k) {
       if (valid[k]) {
-        const double2 v = apply_pose(R00, R01, R10, R11, T0, T1, sx[k], sy[k]);
+        const double2 v = apply_pose(P, sx[k], sy[k]);
         sx[k] = v.x; sy[k] = v.y;
       }
     }
@@ -135,7 +130,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
       }
       // ---- gate, evaluation sums and the Gauss-Newton system at this pose, one reduction:
       // r[0..5] = H (00 01 02 11 12 22), r[6..8] = g, r[9] = inliers, r[10] = sum d^2, r[11] = sum d
-      const double2 c = apply_pose(R00, R01, R10, R11, T0, T1, cax, cay);
+      const double2 c = apply_pose(P, cax, cay);
       double r[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 #pragma unroll
       for (int k = 0; k < S; ++k) {
@@ -146,11 +141,11 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
             const double2 b = load_point(pr.tgt_points, pr.dtype, j);
             const double* cb = a.tgt_cov + j * 3;
             // S = C_B + R C_A R^T, M = S^-1 (closed form)
-            const double u00 = R00 * ca[k][0] + R01 * ca[k][1], u01 = R00 * ca[k][1] + R01 * ca[k][2];
-            const double u10 = R10 * ca[k][0] + R11 * ca[k][1], u11 = R10 * ca[k][1] + R11 * ca[k][2];
-            const double sa = __ldg(cb) + (u00 * R00 + u01 * R01);
-            const double sb = __ldg(cb + 1) + (u00 * R10 + u01 * R11);
-            const double sd = __ldg(cb + 2) + (u10 * R10 + u11 * R11);
+            const double u00 = P.r00 * ca[k][0] + P.r01 * ca[k][1], u01 = P.r00 * ca[k][1] + P.r01 * ca[k][2];
+            const double u10 = P.r10 * ca[k][0] + P.r11 * ca[k][1], u11 = P.r10 * ca[k][1] + P.r11 * ca[k][2];
+            const double sa = __ldg(cb) + (u00 * P.r00 + u01 * P.r01);
+            const double sb = __ldg(cb + 1) + (u00 * P.r10 + u01 * P.r11);
+            const double sd = __ldg(cb + 2) + (u10 * P.r10 + u11 * P.r11);
             const double inv = 1.0 / (sa * sd - sb * sb);
             const double m00 = sd * inv, m01 = -sb * inv, m11 = sa * inv;
             const double rx = sx[k] - c.x, ry = sy[k] - c.y;
@@ -168,11 +163,12 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
       rb ^= 1;
       const double cnt = r[9];
       if (cnt < 0.5) {                                       // nothing inside the gate: stop
-        err = CUDART_INF; rmse = CUDART_INF; inl = 0;
+        err = CUDART_INF; mean_d2 = CUDART_INF; inl = 0;
         break;
       }
-      const double fit = cnt * inv_n, rm = sqrt(r[10] / cnt);
-      err = r[11] / cnt; rmse = rm; inl = (int)(cnt + 0.5);
+      mean_d2 = r[10] / cnt;
+      const double fit = cnt * inv_n, rm = sqrt(mean_d2);
+      err = r[11] / cnt; inl = (int)(cnt + 0.5);
       if (e > 0 && fabs(fit - fit_prev) < op.relative_fitness && fabs(rm - rmse_prev) < op.relative_rmse) break;
       if (iters >= op.max_iterations) break;
       fit_prev = fit; rmse_prev = rm;
@@ -217,32 +213,17 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
         }
       }
       {
-        const double n00 = R00 + (cm1 * R00 - sn * R10), n01 = R01 + (cm1 * R01 - sn * R11);
-        const double n10 = R10 + (sn * R00 + cm1 * R10), n11 = R11 + (sn * R01 + cm1 * R11);
-        const double tx = T0 - c.x, ty = T1 - c.y;
-        const double nt0 = T0 + ((cm1 * tx - sn * ty) + dx), nt1 = T1 + ((sn * tx + cm1 * ty) + dy);
-        R00 = n00; R01 = n01; R10 = n10; R11 = n11; T0 = nt0; T1 = nt1;
+        const double tx = P.tx - c.x, ty = P.ty - c.y;
+        P = Se2{P.r00 + (cm1 * P.r00 - sn * P.r10), P.r01 + (cm1 * P.r01 - sn * P.r11),
+                P.r10 + (sn * P.r00 + cm1 * P.r10), P.r11 + (sn * P.r01 + cm1 * P.r11),
+                P.tx + ((cm1 * tx - sn * ty) + dx), P.ty + ((sn * tx + cm1 * ty) + dy)};
       }
-      c_last = 1.0 + cm1; s_last = sn;
-      t0_last = dx - (cm1 * c.x - sn * c.y);
-      t1_last = dy - (sn * c.x + cm1 * c.y);
+      last = Increment{1.0 + cm1, sn, dx - (cm1 * c.x - sn * c.y), dy - (sn * c.x + cm1 * c.y)};
       ++iters;
     }
   }
 
-  if (tid == 0) {
-    double* pt = out.pose_total + p * 6;
-    pt[0] = R00; pt[1] = R01; pt[2] = R10; pt[3] = R11; pt[4] = T0; pt[5] = T1;
-    if (out.pose_last) {
-      double* pl = out.pose_last + p * 6;
-      pl[0] = c_last; pl[1] = -s_last; pl[2] = s_last; pl[3] = c_last;
-      pl[4] = t0_last; pl[5] = t1_last;
-    }
-    out.error[p] = err;
-    if (out.rmse) out.rmse[p] = rmse;
-    if (out.inliers) out.inliers[p] = inl;
-    out.iterations[p] = iters;
-  }
+  if (tid == 0) write_pair_result(out, p, P, last, err, mean_d2, inl, iters);
   if (out.indices || out.src_final) {
     const bool ran = n > 0 && m > 0;
 #pragma unroll
@@ -252,7 +233,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) gicp_align_kernel(const Gic
         if (out.indices) out.indices[p * pr.src_pitch + i] = (valid[k] && ran) ? idx[k] : -1;
         if (out.src_final) {
           double2 v = make_double2(0.0, 0.0);
-          if (valid[k]) v = ran ? make_double2(sx[k], sy[k]) : apply_pose(R00, R01, R10, R11, T0, T1, sx[k], sy[k]);
+          if (valid[k]) v = ran ? make_double2(sx[k], sy[k]) : apply_pose(P, sx[k], sy[k]);
           reinterpret_cast<double2*>(out.src_final)[p * pr.src_pitch + i] = v;
         }
       }

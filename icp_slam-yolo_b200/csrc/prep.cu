@@ -18,7 +18,7 @@ namespace {
 // ------------------------------------------------------------------------------------
 // kernel: best_fit_transform(A, B) for matched rows (icp.py:5-26), one warp per pair:
 // centroids, centred 2x2 cross-covariance (single pass, each cloud relative to its first point),
-// closed-form proper rotation, t = cB - R cA.
+// closed-form proper rotation, t = cB - R cA (kabsch_increment, icp_step.cuh).
 // ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(32) best_fit_warp_kernel(const KernelArgs a) {
   const int lane = threadIdx.x;
@@ -26,12 +26,12 @@ __global__ void __launch_bounds__(32) best_fit_warp_kernel(const KernelArgs a) {
   const b200icp_problem& pr = a.prob;
   int64_t srow, trow;
   resolve_rows(pr, p, srow, trow);
-  const int ns = pr.src_len ? min(pr.src_len[srow], pr.src_pitch) : pr.src_pitch;
-  const int nt = pr.tgt_len ? min(pr.tgt_len[trow], pr.tgt_pitch) : pr.tgt_pitch;
+  int ns, nt;
+  row_lengths(pr, srow, trow, ns, nt);
   const int n = min(ns, nt);
   double* pose = a.out.pose_total + p * 6;
   if (n <= 0) {
-    if (lane == 0) { pose[0] = 1; pose[1] = 0; pose[2] = 0; pose[3] = 1; pose[4] = 0; pose[5] = 0; }
+    if (lane == 0) se2_store(pose, se2_identity());
     return;
   }
   // each cloud relative to its own first point: the single-pass sums then cancel only as much as
@@ -42,30 +42,14 @@ __global__ void __launch_bounds__(32) best_fit_warp_kernel(const KernelArgs a) {
   for (int i = lane; i < n; i += 32) {
     const double2 s = load_point(pr.src_points, pr.dtype, srow * pr.src_pitch + i);
     const double2 b = load_point(pr.tgt_points, pr.dtype, trow * pr.tgt_pitch + i);
-    const double ax = s.x - oa.x, ay = s.y - oa.y, qx = b.x - o.x, qy = b.y - o.y;
-    r[0] += ax; r[1] += ay; r[2] += qx; r[3] += qy;
-    r[4] = fma(ax, qx, r[4]); r[5] = fma(ax, qy, r[5]);
-    r[6] = fma(ay, qx, r[6]); r[7] = fma(ay, qy, r[7]);
+    add_match(r, s.x - oa.x, s.y - oa.y, b.x - o.x, b.y - o.y);
   }
 #pragma unroll
   for (int q = 0; q < 8; ++q) {
 #pragma unroll
     for (int s = 16; s > 0; s >>= 1) r[q] += __shfl_xor_sync(kFull, r[q], s);
   }
-  if (lane == 0) {
-    const double inv = 1.0 / (double)n;
-    const double max_ = r[0] * inv, may_ = r[1] * inv, mbx = r[2] * inv, mby = r[3] * inv;
-    const double h00 = fma(-r[0], mbx, r[4]), h01 = fma(-r[0], mby, r[5]);
-    const double h10 = fma(-r[1], mbx, r[6]), h11 = fma(-r[1], mby, r[7]);
-    const double num = h01 - h10, den = h00 + h11;
-    const double h2 = fma(num, num, den * den);
-    double cs = 1.0, sn = 0.0;
-    if (h2 > 0.0) { const double rh = rsqrt(h2); cs = den * rh; sn = num * rh; }
-    const double cax = oa.x + max_, cay = oa.y + may_;
-    pose[0] = cs; pose[1] = -sn; pose[2] = sn; pose[3] = cs;
-    pose[4] = (o.x + mbx) - (cs * cax - sn * cay);          // icp.py:25
-    pose[5] = (o.y + mby) - (sn * cax + cs * cay);
-  }
+  if (lane == 0) se2_store(pose, as_se2(kabsch_increment(r, 1.0 / (double)n, oa.x, oa.y, o.x, o.y)));
 }
 
 // ------------------------------------------------------------------------------------
@@ -154,24 +138,6 @@ struct CopyPoint {
 // contiguous segment, thread 0 scans the 1,024 segment totals, every thread rewrites its
 // segment with its prefix.  out[0] = identity, out[k+1] = out[k] o pose[k].
 // ------------------------------------------------------------------------------------
-struct Se2 {
-  double r00, r01, r10, r11, tx, ty;
-};
-__device__ __forceinline__ Se2 se2_identity() { return Se2{1.0, 0.0, 0.0, 1.0, 0.0, 0.0}; }
-__device__ __forceinline__ Se2 se2_load(const double* p) { return Se2{p[0], p[1], p[2], p[3], p[4], p[5]}; }
-__device__ __forceinline__ void se2_store(double* p, const Se2& a) {
-  p[0] = a.r00; p[1] = a.r01; p[2] = a.r10; p[3] = a.r11; p[4] = a.tx; p[5] = a.ty;
-}
-// a o b : first b, then a  (x -> Ra (Rb x + tb) + ta)
-__device__ __forceinline__ Se2 se2_mul(const Se2& a, const Se2& b) {
-  Se2 c;
-  c.r00 = a.r00 * b.r00 + a.r01 * b.r10; c.r01 = a.r00 * b.r01 + a.r01 * b.r11;
-  c.r10 = a.r10 * b.r00 + a.r11 * b.r10; c.r11 = a.r10 * b.r01 + a.r11 * b.r11;
-  c.tx = a.r00 * b.tx + a.r01 * b.ty + a.tx;
-  c.ty = a.r10 * b.tx + a.r11 * b.ty + a.ty;
-  return c;
-}
-
 __global__ void __launch_bounds__(1024) chain_poses_kernel(const double* __restrict__ poses, int64_t n,
                                                            double* __restrict__ out) {
   __shared__ double seg[1024][6];

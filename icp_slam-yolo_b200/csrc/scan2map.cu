@@ -29,8 +29,9 @@
 //   s2m_update_kernel   waits for the flags of all ranks (system-scope acquire), then per point
 //                       the global winner (smaller distance, then lower global index), centred
 //                       sums in a fixed order (per-CTA partials, last CTA adds them by CTA index),
-//                       closed-form pose, convergence: bit-identical on every rank, so no second
-//                       collective is needed.  The increment is applied by the next search.
+//                       closed-form pose (icp_step.cuh), convergence: bit-identical on every
+//                       rank, so no second collective is needed.  The increment is applied by
+//                       the next search.
 // A skipped chunk is PROVEN farther from the point than its nearest neighbour, so indices equal
 // the float64 brute force (KD-tree) result.  On the benchmark map (16.7 M points along ~100 m of
 // wall) a scan point meets ~7 chunks instead of 16,384.
@@ -272,19 +273,17 @@ __global__ void __launch_bounds__(32) s2m_super_kernel(const double* __restrict_
 __global__ void __launch_bounds__(256) s2m_init_kernel(const void* scan, int dtype, int n,
                                                        const double* init_pose, double* src64,
                                                        double* prev_nn, b200icp_s2m_state* state) {
-  double R00 = 1, R01 = 0, R10 = 0, R11 = 1, T0 = 0, T1 = 0;
-  if (init_pose) { R00 = init_pose[0]; R01 = init_pose[1]; R10 = init_pose[2]; R11 = init_pose[3]; T0 = init_pose[4]; T1 = init_pose[5]; }
+  const Se2 pose = load_init_pose(init_pose, 0);
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const double2 q = load_point(scan, dtype, i);
-    src64[2 * i] = init_pose ? R00 * q.x + R01 * q.y + T0 : q.x;
-    src64[2 * i + 1] = init_pose ? R10 * q.x + R11 * q.y + T1 : q.y;
+    const double2 v = init_pose ? apply(pose, q) : q;
+    src64[2 * i] = v.x;
+    src64[2 * i + 1] = v.y;
     if (prev_nn) { prev_nn[2 * i] = CUDART_NAN; prev_nn[2 * i + 1] = CUDART_NAN; }   // "no previous neighbour"
   }
   if (blockIdx.x == 0 && threadIdx.x == 0) {
-    state->pose_total[0] = R00; state->pose_total[1] = R01; state->pose_total[2] = R10;
-    state->pose_total[3] = R11; state->pose_total[4] = T0; state->pose_total[5] = T1;
-    state->pose_last[0] = 1; state->pose_last[1] = 0; state->pose_last[2] = 0;
-    state->pose_last[3] = 1; state->pose_last[4] = 0; state->pose_last[5] = 0;
+    se2_store(state->pose_total, pose);
+    se2_store(state->pose_last, se2_identity());
     state->error = CUDART_INF; state->mean_d2 = CUDART_INF; state->prev_error = 0.0;   // icp.py:33
     state->iterations = 0; state->inliers = 0; state->done = (n <= 0) ? 1 : 0; state->applied = 0;
   }
@@ -292,8 +291,7 @@ __global__ void __launch_bounds__(256) s2m_init_kernel(const void* scan, int dty
 
 // src <- R_last src + t_last for the increment an update left pending (icp.py:45)
 __device__ __forceinline__ double2 apply_pending(const b200icp_s2m_state* st, double2 s) {
-  const double cs = st->pose_last[0], sn = st->pose_last[2], tx = st->pose_last[4], ty = st->pose_last[5];
-  return make_double2(cs * s.x - sn * s.y + tx, sn * s.x + cs * s.y + ty);
+  return apply(Increment{st->pose_last[0], st->pose_last[2], st->pose_last[4], st->pose_last[5]}, s);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -792,11 +790,7 @@ __global__ void __launch_bounds__(kUpdateThreads) s2m_update_kernel(const Update
     if (!use_gate || dist < a.max_corr_dist) {
       double2 s = make_double2(a.src64[2 * i], a.src64[2 * i + 1]);
       if (pending) s = apply_pending(st, s);
-      const double ax = s.x - o.x, ay = s.y - o.y;
-      const double qx = w.z - o.x, qy = w.w - o.y;
-      r[0] += ax; r[1] += ay; r[2] += qx; r[3] += qy;
-      r[4] = fma(ax, qx, r[4]); r[5] = fma(ax, qy, r[5]);
-      r[6] = fma(ay, qx, r[6]); r[7] = fma(ay, qy, r[7]);
+      add_match(r, s.x - o.x, s.y - o.y, w.z - o.x, w.w - o.y);
       r[8] += dist; r[9] += w.x; r[10] += 1.0;
     }
   }
@@ -844,25 +838,10 @@ __global__ void __launch_bounds__(kUpdateThreads) s2m_update_kernel(const Update
     return;
   }
   const double inv = 1.0 / cnt;
-  const double max_ = tot[0] * inv, may_ = tot[1] * inv, mbx = tot[2] * inv, mby = tot[3] * inv;
   const double mean_error = tot[8] * inv;                          // icp.py:48
-  const double h00 = fma(-tot[0], mbx, tot[4]), h01 = fma(-tot[0], mby, tot[5]);
-  const double h10 = fma(-tot[1], mbx, tot[6]), h11 = fma(-tot[1], mby, tot[7]);
-  const double num = h01 - h10, den = h00 + h11;
-  const double h2 = fma(num, num, den * den);
-  double cs = 1.0, sn = 0.0;
-  if (h2 > 0.0) { const double rh = rsqrt(h2); cs = den * rh; sn = num * rh; }
-  const double cax = o.x + max_, cay = o.y + may_;
-  const double tx = (o.x + mbx) - (cs * cax - sn * cay);            // icp.py:25
-  const double ty = (o.y + mby) - (sn * cax + cs * cay);
-  const double R00 = st->pose_total[0], R01 = st->pose_total[1];
-  const double R10 = st->pose_total[2], R11 = st->pose_total[3];
-  const double T0 = st->pose_total[4], T1 = st->pose_total[5];
-  st->pose_total[0] = cs * R00 - sn * R10; st->pose_total[1] = cs * R01 - sn * R11;
-  st->pose_total[2] = sn * R00 + cs * R10; st->pose_total[3] = sn * R01 + cs * R11;
-  st->pose_total[4] = cs * T0 - sn * T1 + tx; st->pose_total[5] = sn * T0 + cs * T1 + ty;
-  st->pose_last[0] = cs; st->pose_last[1] = -sn; st->pose_last[2] = sn;
-  st->pose_last[3] = cs; st->pose_last[4] = tx; st->pose_last[5] = ty;
+  const Increment d = kabsch_increment(tot, inv, o.x, o.y, o.x, o.y);
+  se2_store(st->pose_total, compose(d, se2_load(st->pose_total)));
+  se2_store(st->pose_last, as_se2(d));
   st->error = mean_error; st->mean_d2 = tot[9] * inv; st->inliers = (int)(cnt + 0.5);
   const int it = st->iterations + 1;
   st->iterations = it;                                               // > applied: the increment is pending

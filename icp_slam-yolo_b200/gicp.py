@@ -16,18 +16,19 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .registration import (AlignResult, ScanTable, _check_out, _check_pairs, _default_pairs, _init_pose_ptr,
-                           _outputs, _problem, _ptr, _require_cuda, _stream_ptr, alloc_outputs)
+from .registration import (_DTYPES, AlignResult, ScanTable, _check_out, _check_pairs, _default_pairs, _init_pose_ptr,
+                           _outputs, _problem, _ptr, _registration_4x4, _require_cuda, _rmse_pose, _stream_ptr,
+                           alloc_outputs)
 
 
 def estimate_covariances(table: ScanTable, k: int = 20, epsilon: float = 1e-3, stream=None) -> torch.Tensor:
     """Regularised covariance of every point from its k nearest points in the same row:
     float64 [rows, pitch, 3] (cxx, cxy, cyy), zeros past each row's length.  3 <= k <= 32."""
     out = torch.empty((table.rows, table.pitch, 3), dtype=torch.float64, device=table.points.device)
-    dtype = _cabi.F64 if table.points.dtype == torch.float64 else _cabi.F32
     with torch.cuda.device(table.points.device):
         rc = _cabi.lib().b200icp_estimate_covariances(_ptr(table.points), _ptr(table.lengths), table.rows, table.pitch,
-                                                      dtype, int(k), float(epsilon), _ptr(out), _stream_ptr(stream))
+                                                      _DTYPES[table.points.dtype], int(k), float(epsilon), _ptr(out),
+                                                      _stream_ptr(stream))
     _cabi.check(rc, "b200icp_estimate_covariances")
     return out
 
@@ -90,14 +91,6 @@ def gicp_consecutive(table: ScanTable, k: int = 20, epsilon: float = 1e-3, *, ma
                       out=out, stream=stream, **kw)
 
 
-def _device_points(p) -> torch.Tensor:
-    if isinstance(p, torch.Tensor):
-        t = p[:, :2].to(device="cuda", dtype=torch.float64)
-    else:
-        t = torch.from_numpy(np.ascontiguousarray(np.asarray(p, dtype=np.float64)[:, :2])).cuda()
-    return t.contiguous()
-
-
 def registration_gicp(points1, points2, threshold: float = 200.0, voxel_size: Optional[float] = None,
                       trans_init=None, max_iteration: int = 50, k: int = 20, epsilon: float = 1e-3,
                       relative_fitness: float = 1e-6, relative_rmse: float = 1e-6):
@@ -108,22 +101,14 @@ def registration_gicp(points1, points2, threshold: float = 200.0, voxel_size: Op
     and the voxel filter of both clouds (gicp_lidar.py:20-21).  NumPy arrays or CUDA tensors,
     (N, 2) or (N, 3); one device-to-host read.  rmse is +inf when no pair lies within ``threshold``.
     """
-    if len(points1) < 10 or len(points2) < 10:
-        return float("inf"), np.eye(4)
-    p1, p2 = _device_points(points1), _device_points(points2)
-    if voxel_size:
-        from .mapping import voxel_down_sample
-        p1, p2 = voxel_down_sample(p1, voxel_size), voxel_down_sample(p2, voxel_size)
-    s, t = ScanTable(p1[None].contiguous()), ScanTable(p2[None].contiguous())
-    init = None
-    if trans_init is not None:
-        from .icp import _pose6
-        init = _pose6(np.asarray(trans_init))
-    res = gicp_pairs(s, t, estimate_covariances(s, k, epsilon), estimate_covariances(t, k, epsilon), n_pairs=1,
-                     max_iterations=max_iteration, max_corr_dist=threshold, init_pose=init,
-                     relative_fitness=relative_fitness, relative_rmse=relative_rmse)
-    host = torch.cat([res.pose_total[0], res.rmse]).cpu().numpy()       # one device-to-host read
-    T = np.eye(4)
-    T[:2, :2] = host[:4].reshape(2, 2)
-    T[:2, 3] = host[4:6]
-    return float(host[6]), T
+    def solve(p1, p2):
+        s, t = ScanTable(p1[None].contiguous()), ScanTable(p2[None].contiguous())
+        init = None
+        if trans_init is not None:
+            from .icp import _pose6
+            init = _pose6(np.asarray(trans_init))
+        return _rmse_pose(gicp_pairs(s, t, estimate_covariances(s, k, epsilon), estimate_covariances(t, k, epsilon),
+                                     n_pairs=1, max_iterations=max_iteration, max_corr_dist=threshold, init_pose=init,
+                                     relative_fitness=relative_fitness, relative_rmse=relative_rmse))
+
+    return _registration_4x4(points1, points2, voxel_size, solve)

@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .registration import ScanTable, align_pairs, best_fit, nn_search
+from .registration import ScanTable, _registration_4x4, _rmse_pose, align_pairs, best_fit, nn_search
 
 
 @dataclass
@@ -203,33 +203,15 @@ def registration_p2p(points1, points2, threshold: float = 200.0, voxel_size: Opt
     ``points1`` / ``points2`` may be NumPy arrays or CUDA tensors ((N, 2) or (N, 3)); tensors stay
     on the device from the voxel grid to the pose (the SLAM loop passes its map that way).
     """
-    if len(points1) < 10 or len(points2) < 10:
-        return float("inf"), np.eye(4)
+    def solve(p1, p2):
+        lib = _cabi.lib()
+        if p1.shape[0] > lib.b200icp_max_src_pitch() or p2.shape[0] > lib.b200icp_max_tgt_pitch():
+            o = _icp_full_large(p1.cpu().numpy(), p2.cpu().numpy(), max_iteration, tolerance,
+                                None if trans_init is None else np.asarray(trans_init), threshold)
+            return o.rmse, o.R, o.t
+        return _rmse_pose(align_pairs(ScanTable(p1[None].contiguous()), ScanTable(p2[None].contiguous()), n_pairs=1,
+                                      max_iterations=max_iteration, tolerance=tolerance,
+                                      init_pose=None if trans_init is None else _pose6(np.asarray(trans_init)),
+                                      max_corr_dist=threshold))
 
-    def dev(p):
-        if isinstance(p, torch.Tensor):
-            t = p[:, :2].to(device="cuda", dtype=torch.float64)
-        else:
-            t = torch.from_numpy(np.ascontiguousarray(np.asarray(p, dtype=np.float64)[:, :2])).cuda()
-        return t.contiguous()
-
-    p1, p2 = dev(points1), dev(points2)
-    if voxel_size:                       # gicp_lidar.py:20-21: both clouds are down-sampled first
-        from .mapping import voxel_down_sample
-        p1, p2 = voxel_down_sample(p1, voxel_size), voxel_down_sample(p2, voxel_size)
-    lib = _cabi.lib()
-    if p1.shape[0] > lib.b200icp_max_src_pitch() or p2.shape[0] > lib.b200icp_max_tgt_pitch():
-        o = _icp_full_large(p1.cpu().numpy(), p2.cpu().numpy(), max_iteration, tolerance,
-                            None if trans_init is None else np.asarray(trans_init), threshold)
-        rmse, R, t = o.rmse, o.R, o.t
-    else:
-        res = align_pairs(ScanTable(p1[None].contiguous()), ScanTable(p2[None].contiguous()), n_pairs=1,
-                          max_iterations=max_iteration, tolerance=tolerance,
-                          init_pose=None if trans_init is None else _pose6(np.asarray(trans_init)),
-                          max_corr_dist=threshold)
-        host = torch.cat([res.pose_total[0], res.rmse]).cpu().numpy()       # one device-to-host read
-        R, t, rmse = host[:4].reshape(2, 2), host[4:6], float(host[6])
-    T = np.eye(4)
-    T[:2, :2] = R
-    T[:2, 3] = t
-    return rmse, T
+    return _registration_4x4(points1, points2, voxel_size, solve)

@@ -236,6 +236,38 @@ def _outputs(out: "AlignResult") -> "_cabi.Outputs":
     return o
 
 
+def _device_points(p) -> torch.Tensor:
+    """NumPy array or tensor, (N, 2) or (N, 3) -> contiguous float64 (N, 2) CUDA tensor."""
+    if isinstance(p, torch.Tensor):
+        t = p[:, :2].to(device="cuda", dtype=torch.float64)
+    else:
+        t = torch.from_numpy(np.ascontiguousarray(np.asarray(p, dtype=np.float64)[:, :2])).cuda()
+    return t.contiguous()
+
+
+def _registration_4x4(points1, points2, voxel_size, solve):
+    """The Open3D-shaped ``(rmse, T4x4)`` call around ``solve(p1, p2) -> (rmse, R, t)``: the ``< 10``
+    points guard (gicp_lidar.py:13-15), both clouds on the device as float64 (N, 2), and the voxel
+    filter of both clouds (gicp_lidar.py:20-21)."""
+    if len(points1) < 10 or len(points2) < 10:
+        return float("inf"), np.eye(4)
+    p1, p2 = _device_points(points1), _device_points(points2)
+    if voxel_size:
+        from .mapping import voxel_down_sample
+        p1, p2 = voxel_down_sample(p1, voxel_size), voxel_down_sample(p2, voxel_size)
+    rmse, R, t = solve(p1, p2)
+    T = np.eye(4)
+    T[:2, :2] = R
+    T[:2, 3] = t
+    return rmse, T
+
+
+def _rmse_pose(res: "AlignResult"):
+    """(rmse, R, t) of pair 0, in one device-to-host read."""
+    host = torch.cat([res.pose_total[0], res.rmse]).cpu().numpy()
+    return float(host[6]), host[:4].reshape(2, 2), host[4:6]
+
+
 def nn_search(src: ScanTable, tgt: ScanTable, *, n_pairs: Optional[int] = None,
               pairing: str = "rowwise", src_row=None, tgt_row=None, first_pair: int = 0,
               want_dist2: bool = True, out_idx=None, out_dist2=None, validate_rows: bool = False,

@@ -7,7 +7,9 @@ source file name) and without the parameter list; OLD=NEW pairs match a renamed 
 kernel of BASE it prints "same", "differs" (the instruction stream or REG / STACK / SHARED / LOCAL),
 or "missing"; kernels only in NEW are listed as "new".  A differing kernel is marked "resources only"
 when its instructions are identical, and "params only" when they match once the constant-bank
-(kernel parameter) offsets are masked.  Exit code 1 if any kernel of BASE differs or is missing.
+(kernel parameter) offsets are masked.  Under every other "differs" line it prints the resources
+that changed and the per-opcode count changes (opcodes without their modifiers: DFMA, MUFU, ...).
+Exit code 1 if any kernel of BASE differs or is missing.
 """
 import collections
 import re
@@ -50,6 +52,18 @@ def masked(body):
     return [re.sub(r"c\[0x0\]\[0x[0-9a-f]+\]", "c[0x0][P]", ins) for ins in body]
 
 
+def opcodes(body):
+    return collections.Counter(re.sub(r"^@!?U?P\w+\s+", "", ins).split()[0].split(".")[0] for ins in body)
+
+
+def delta(body, res, body2, res2):
+    """What changed between two versions of a kernel: resources, then opcode counts."""
+    out = [f"{k} {a} -> {b}" for k, a, b in zip(RES, res, res2) if a != b]
+    c, c2 = opcodes(body), opcodes(body2)
+    out += [f"{op} {c2[op] - c[op]:+d}" for op in sorted(set(c) | set(c2)) if c[op] != c2[op]]
+    return ", ".join(out) or "same opcode counts and resources"
+
+
 def main():
     base, new = kernels(sys.argv[1]), kernels(sys.argv[2])
     renamed = dict(a.split("=", 1) for a in sys.argv[3:])
@@ -73,6 +87,8 @@ def main():
                 else:
                     status = "differs"
             print(f"{status:9s} {name}" + (f" -> {twin}" if twin != name else "") + f"  ({len(body)} instructions)")
+            if status == "differs" and len(new[twin]) == 1:
+                print("          " + delta(body, res, *new[twin][0]))
     for name in sorted(set(new) - seen):
         print(f"new       {name}")
     print(f"{sum(len(v) for v in base.values())} base kernels, {bad} differ or are missing")
