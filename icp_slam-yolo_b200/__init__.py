@@ -11,6 +11,8 @@ from .registration import (AlignResult, ScanTable, align_pairs, alloc_outputs,  
                            best_fit, ffma_probe, nn_search, polar_to_cartesian)
 from .odometry import align_consecutive, chain_poses         # noqa: F401
 from .gicp import estimate_covariances, gicp_consecutive, gicp_pairs, registration_gicp   # noqa: F401
+from .pose_graph import (PoseGraph, PoseGraphResult, close_loops, information_matrices,   # noqa: F401
+                         loop_candidates, optimize_pose_graph)
 from .sharding import shard_range, triangle_pair, triangle_pair_count   # noqa: F401
 from .scan_to_map import MapShard, ScanToMap, ScanToMapResult, scan_to_map_icp   # noqa: F401
 from .mapping import crop_local_map, remove_dynamic_points, voxel_down_sample   # noqa: F401
@@ -26,4 +28,5 @@ __all__ = [
     "scan_to_map_icp", "crop_local_map", "remove_dynamic_points", "voxel_down_sample",
     "OccupancyGrid", "map_io", "hostmem", "OfflineSlam", "SlamConfig",
     "estimate_covariances", "gicp_pairs", "gicp_consecutive", "registration_gicp",
+    "loop_candidates", "information_matrices", "PoseGraph", "PoseGraphResult", "optimize_pose_graph", "close_loops",
 ]

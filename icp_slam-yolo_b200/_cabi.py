@@ -94,6 +94,34 @@ class OccGrid(C.Structure):
     ]
 
 
+class PoseGraphBatch(C.Structure):
+    _fields_ = [
+        ("n_graphs", C.c_int32), ("reserved", C.c_int32),
+        ("node_offset", C.c_void_p), ("edge_offset", C.c_void_p), ("fixed_node", C.c_void_p),
+        ("poses_in", C.c_void_p), ("edge_i", C.c_void_p), ("edge_j", C.c_void_p),
+        ("meas", C.c_void_p), ("info", C.c_void_p),
+    ]
+
+
+class PoseGraphOptions(C.Structure):
+    _fields_ = [
+        ("max_iterations", C.c_int32), ("pcg_max_iterations", C.c_int32),
+        ("tolerance", C.c_double), ("pcg_tolerance", C.c_double), ("damping", C.c_double),
+    ]
+
+
+class PoseGraphOutputs(C.Structure):
+    _fields_ = [
+        ("poses", C.c_void_p), ("chi2_initial", C.c_void_p), ("chi2_final", C.c_void_p),
+        ("iterations", C.c_void_p), ("pcg_iterations", C.c_void_p), ("status", C.c_void_p),
+        ("isolated", C.c_void_p), ("anchored", C.c_void_p),
+    ]
+
+
+PG_STATUS_NAMES = {0: "converged", 1: "max_iterations", 2: "pcg_limit", 3: "non_finite", 4: "bad_edge",
+                   5: "pcg_breakdown"}
+
+
 # symbol -> (restype, argtypes); must list EVERY function include/b200icp.h declares
 SYMBOLS = {
     "b200icp_version": (C.c_int, []),
@@ -141,6 +169,18 @@ SYMBOLS = {
     "b200icp_peer_open": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "b200icp_peer_close": (C.c_int, [C.c_void_p]),
     "b200icp_peer_free": (C.c_int, [C.c_void_p]),
+    "b200icp_loop_candidates": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_double, C.c_int64, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200icp_information_batch": (C.c_int, [C.POINTER(Problem), C.c_int64, C.c_void_p, C.c_void_p, C.c_double,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200icp_loop_edges": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200icp_odometry_edges": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200icp_pose_graph_workspace_bytes": (C.c_int64, [C.POINTER(PoseGraphBatch)]),
+    "b200icp_pose_graph_optimize": (C.c_int, [C.POINTER(PoseGraphBatch), C.POINTER(PoseGraphOptions),
+                                              C.POINTER(PoseGraphOutputs), C.c_void_p, C.c_int64, C.c_void_p]),
 }
 
 _lib = None

@@ -45,7 +45,7 @@ int check_launch(const char* what, ...) {
   return set_error(B200ICP_ERR_CUDA, "%s: %s", buf, cudaGetErrorString(e));
 }
 
-int check_problem(const b200icp_problem* pr, int64_t n_pairs) {
+int check_problem(const b200icp_problem* pr, int64_t n_pairs, bool pitch_limit) {
   if (!pr) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "problem is NULL");
   if (n_pairs < 0) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "n_pairs < 0");
   if (!pr->src_points || !pr->tgt_points)
@@ -63,7 +63,7 @@ int check_problem(const b200icp_problem* pr, int64_t n_pairs) {
     if (rows < 2 || pr->first_pair < 0 || pr->first_pair + n_pairs > rows * (rows - 1) / 2)
       return set_error(B200ICP_ERR_INVALID_ARGUMENT, "TRIANGLE pairing: pair range outside n_rows*(n_rows-1)/2");
   }
-  if (pr->src_pitch > kMaxSrcPitch || pr->tgt_pitch > kMaxTgtPitch)
+  if (pitch_limit && (pr->src_pitch > kMaxSrcPitch || pr->tgt_pitch > kMaxTgtPitch))
     return set_error(B200ICP_ERR_UNSUPPORTED_SHAPE, "pitch beyond the fused per-pair kernel (src <= 1024, tgt <= 4096)");
   if (n_pairs > 0x7fffffffLL) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "n_pairs > 2^31-1 per call");
   return B200ICP_OK;

@@ -459,6 +459,143 @@ int b200icp_occ_filter_points(const void* points, int32_t dtype, int32_t cols, i
                               float free_threshold, int64_t* kept_index, int64_t* count_out,
                               int64_t* scratch, void* stream);
 
+/* ---- loop closure: candidates, edge information, graph edges and a batched SE(2) pose-graph
+ * optimiser (DESIGN.md §4.9).  The reference has no loop closure; oracle/pose_graph_oracle.py
+ * defines every result below (parity-unpinned).
+ *
+ * Conventions
+ *   - A pose is [R00 R01 R10 R11 tx ty] (float64).  The graph state X_k is the global pose of scan k,
+ *     as b200icp_chain_poses returns it.
+ *   - For a pair with source row j and target row i, pose_total maps points of j into the frame of i:
+ *     it is the measurement Z_ij ~ X_i^-1 X_j.  Odometry pair p is (i, j) = (p, p + 1); a loop edge
+ *     is (i, j) with i < j.
+ *   - Edge error e_ij = t2v(Z_ij^-1 (X_i^-1 X_j)) in the order (x, y, theta), theta = atan2 of the
+ *     rotation, wrapped to (-pi, pi]; the Jacobians are the standard SE(2) ones (Grisetti et al.,
+ *     "A Tutorial on Graph-Based SLAM", §IV): with S = Rz^T Ri^T and v = Rz^T dRi^T/dtheta (tj - ti),
+ *     A = [[-S, v], [0 0 -1]], B = [[S, 0], [0 0 1]].  chi2 = sum e^T W e.
+ *   - Information W is stored as its upper triangle [6] = (xx, xy, xt, yy, yt, tt).
+ *   - The step x_k of node k is applied as X_k <- X_k (+) x_k: t += (x0, x1), R <- R R(x2).
+ *   - One node per graph is held fixed (the gauge): its row and column are eliminated.
+ */
+
+/*
+ * Loop candidates from a trajectory.  Pairs (i < j) of the n poses are visited in the linear order
+ * of B200ICP_PAIR_TRIANGLE; a pair is kept when j - i >= min_gap and
+ * d^2 = (tx_i - tx_j)^2 + (ty_i - ty_j)^2 <= radius * radius, each product and sum rounded on its own
+ * (as the local-map crop of b200icp_select_points rounds it).  The k-th kept pair writes
+ * src_row[k] = j, tgt_row[k] = i (int32, ready for B200ICP_PAIR_EXPLICIT) and rel_pose[k][6] =
+ * X_i^-1 X_j = (Ri^T Rj, Ri^T (tj - ti)), every product and sum rounded on its own (ready for
+ * init_pose).  *count_out (device int64) is the number of kept pairs; only the first `capacity` are
+ * written.  scratch: int64[ceil(n (n - 1) / 2 / 1024) + 1].  min_gap >= 1, radius >= 0, n <= 65536.
+ */
+int b200icp_loop_candidates(const double* poses, int64_t n, int64_t min_gap, double radius, int64_t capacity,
+                            int32_t* src_row, int32_t* tgt_row, double* rel_pose, int64_t* count_out,
+                            int64_t* scratch, void* stream);
+
+/*
+ * Information matrix of each aligned pair: the 2D analogue of Open3D's
+ * get_information_matrix_from_point_clouds.  Per pair (one warp): every source point i < len with
+ * indices[p][i] >= 0 is moved by pose[p] (apply() of icp_step.cuh), kept when it passes the gate of
+ * b200icp_align_batch (max_corr_dist <= 0 or +inf: no gate; else distance < max_corr_dist) to its
+ * matched target q, and adds G^T G, G = [[1, 0, -q_y], [0, 1, q_x]] (q in the target frame).
+ * Summation order: lane l adds the points l, l + 32, l + 64, ... in that order (count, -q_y, q_x and
+ * q_x * q_x + q_y * q_y, each product and sum rounded on its own); then v += shfl_xor(v, o) for
+ * o = 16, 8, 4, 2, 1.  info_out[p][6] = (n, 0, -sum q_y, n, sum q_x, sum |q|^2); inliers_out
+ * (may be NULL) = n.  The indices of b200icp_align_batch are those of its last search, made before
+ * the last update (the reference's lag, quirk Q2); those of b200icp_gicp_batch are at the final pose.
+ */
+int b200icp_information_batch(const b200icp_problem* prob, int64_t n_pairs, const double* pose,
+                              const int32_t* indices, double max_corr_dist, double* info_out, int32_t* inliers_out,
+                              void* stream);
+
+/*
+ * Loop edges from verified candidates: pair p is accepted when rmse[p] is finite and <= max_rmse and
+ * fitness = inliers[p] / n_src >= min_fitness (n_src = min(src_len[src_row[p]], src_pitch), or
+ * src_pitch when src_len is NULL; fitness 0 when n_src = 0).  The k-th accepted pair writes
+ * edge_i[k] = tgt_row[p], edge_j[k] = src_row[p], meas[k] = pose_total[p], info_out[k] = info[p]
+ * (identity when info is NULL).  *count_out (device int64) = accepted pairs.
+ * scratch: int64[ceil(n_pairs / 1024) + 1].
+ */
+int b200icp_loop_edges(int64_t n_pairs, const double* pose_total, const double* rmse, const int32_t* inliers,
+                       const int32_t* src_len, int32_t src_pitch, const int32_t* src_row, const int32_t* tgt_row,
+                       const double* info, double min_fitness, double max_rmse, int32_t* edge_i, int32_t* edge_j,
+                       double* meas, double* info_out, int64_t* count_out, int64_t* scratch, void* stream);
+
+/*
+ * Odometry edges from a sequence-odometry result: pair p gives (p, p + 1, pose_total[p], info[p]);
+ * pairs with iterations[p] == 0 or error[p] == +inf are dropped (n_pairs - *count_out of them).
+ */
+int b200icp_odometry_edges(int64_t n_pairs, const double* pose_total, const double* error, const int32_t* iterations,
+                           const double* info, int32_t* edge_i, int32_t* edge_j, double* meas, double* info_out,
+                           int64_t* count_out, int64_t* scratch, void* stream);
+
+/*
+ * Batched SE(2) pose-graph optimisation, one CTA per graph.  Graph g owns nodes
+ * [node_offset[g], node_offset[g + 1]) of poses_in and edges [edge_offset[g], edge_offset[g + 1]);
+ * edge_i / edge_j are indices local to the graph.  Limits: <= 65,536 nodes and <= 2^20 edges per
+ * graph (status 2 otherwise), fewer than 2^31 nodes and 2^30 edges per call.
+ * Per graph: set-up once per call (block-CSR of H: each node's edge slots in ascending edge order,
+ * by a stable radix sort); then Gauss-Newton on the device: linearise (one thread per edge writes
+ * A'WA, A'WB, B'WB, A'We, B'We and e'We to slots owned by the edge), assemble (each node adds its slots
+ * in CSR order, + damping on the diagonal), solve H x = -b by PCG with block-Jacobi (3x3 inverse)
+ * preconditioning in float64, stopping when r'M^-1 r <= pcg_tolerance^2 * r0'M^-1 r0 or after
+ * pcg_max_iterations; dot products are fixed-order CTA reductions, so a graph's result does not
+ * depend on the other graphs of the launch; apply the step and re-linearise.  Stops when
+ * |chi2_prev - chi2| <= tolerance * chi2_prev, chi2 == 0, or after max_iterations steps.
+ * A node that no edge touches gets an identity block and no step (it keeps its pose bit for bit) and
+ * is counted in `isolated`.  The gauge node is eliminated and keeps its pose; so does the lowest-index
+ * node of every other connected component (e.g. the part of a trajectory after a dropped odometry pair
+ * that no loop bridges), counted in `anchored`.  H therefore has no null space.
+ */
+typedef struct b200icp_pose_graph_batch {
+  int32_t n_graphs;
+  int32_t reserved;
+  const int64_t* node_offset;  /* HOST [n_graphs + 1], node_offset[0] = 0                        */
+  const int64_t* edge_offset;  /* HOST [n_graphs + 1], edge_offset[0] = 0                        */
+  const int32_t* fixed_node;   /* HOST [n_graphs] local gauge node, or NULL = node 0 of every graph */
+  const double* poses_in;      /* [nodes][6]                                                       */
+  const int32_t* edge_i;       /* [edges]                                                          */
+  const int32_t* edge_j;       /* [edges]                                                          */
+  const double* meas;          /* [edges][6] Z_ij                                                  */
+  const double* info;          /* [edges][6] upper triangle of W                                   */
+} b200icp_pose_graph_batch;
+
+typedef struct b200icp_pose_graph_options {
+  int32_t max_iterations;      /* Gauss-Newton steps                                               */
+  int32_t pcg_max_iterations;  /* per step                                                         */
+  double tolerance;            /* relative chi2 change                                             */
+  double pcg_tolerance;        /* relative preconditioned residual                                 */
+  double damping;              /* >= 0, added to the diagonal of H (Levenberg)                     */
+} b200icp_pose_graph_options;
+
+typedef enum b200icp_pose_graph_status {
+  B200ICP_PG_CONVERGED = 0,        /* relative chi2 change within tolerance (or chi2 = 0)          */
+  B200ICP_PG_MAX_ITERATIONS = 1,   /* max_iterations steps without converging                      */
+  B200ICP_PG_PCG_LIMIT = 2,        /* some PCG solve stopped at pcg_max_iterations (steps applied)  */
+  B200ICP_PG_NON_FINITE = 3,       /* chi2 or a step not finite: stopped, the last step not applied */
+  B200ICP_PG_BAD_EDGE = 4,         /* an edge endpoint outside the graph or i == j: poses unchanged */
+  B200ICP_PG_PCG_BREAKDOWN = 5     /* p'Hp of a PCG iteration not finite and positive: stopped, that
+                                      step not applied                                             */
+} b200icp_pose_graph_status;
+
+/* Every pointer except poses and status may be NULL. */
+typedef struct b200icp_pose_graph_outputs {
+  double* poses;               /* [nodes][6] optimised (may not alias poses_in)                    */
+  double* chi2_initial;        /* [n_graphs]                                                       */
+  double* chi2_final;          /* [n_graphs]                                                       */
+  int32_t* iterations;         /* [n_graphs] Gauss-Newton steps applied                            */
+  int32_t* pcg_iterations;     /* [n_graphs] PCG iterations over all steps                         */
+  int32_t* status;             /* [n_graphs] b200icp_pose_graph_status                             */
+  int32_t* isolated;           /* [n_graphs] nodes other than the gauge that no edge touches       */
+  int32_t* anchored;           /* [n_graphs] components without the gauge, each held at its lowest node */
+} b200icp_pose_graph_outputs;
+
+/* Device workspace of b200icp_pose_graph_optimize for this batch (-1 on bad arguments). */
+int64_t b200icp_pose_graph_workspace_bytes(const b200icp_pose_graph_batch* graphs);
+int b200icp_pose_graph_optimize(const b200icp_pose_graph_batch* graphs, const b200icp_pose_graph_options* opt,
+                                const b200icp_pose_graph_outputs* out, void* workspace, int64_t workspace_bytes,
+                                void* stream);
+
 /*
  * FP32 FFMA throughput probe used as the roofline denominator of the NN phase
  * (MEASURED_PEAKS.json carries no FP32 figure).  Launches one kernel doing
