@@ -8,6 +8,9 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <mutex>
+#include <set>
+#include <utility>
 
 #include "launch.cuh"
 
@@ -43,6 +46,23 @@ int check_launch(const char* what, ...) {
   vsnprintf(buf, sizeof(buf), what, ap);
   va_end(ap);
   return set_error(B200ICP_ERR_CUDA, "%s: %s", buf, cudaGetErrorString(e));
+}
+
+int opt_in_dynamic_smem(const void* kern, int bytes) {
+  static std::mutex mu;
+  static std::set<std::pair<const void*, int>> opted_in;
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "cudaGetDevice: %s", cudaGetErrorString(e));
+  std::lock_guard<std::mutex> lock(mu);
+  const std::pair<const void*, int> key(kern, dev);
+  if (opted_in.count(key)) return B200ICP_OK;
+  if (bytes < 0) cudaDeviceGetAttribute(&bytes, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e != cudaSuccess)
+    return set_error(B200ICP_ERR_CUDA, "cudaFuncSetAttribute(%d bytes of dynamic smem): %s", bytes, cudaGetErrorString(e));
+  opted_in.insert(key);
+  return B200ICP_OK;
 }
 
 int check_problem(const b200icp_problem* pr, int64_t n_pairs, bool pitch_limit) {

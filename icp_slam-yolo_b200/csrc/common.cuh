@@ -23,6 +23,9 @@ int set_error(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3
 // B200ICP_OK if no CUDA error is pending, else B200ICP_ERR_CUDA with the message
 // "<what>: <CUDA error string>" (`what` is printf-style).
 int check_launch(const char* what, ...) __attribute__((format(printf, 1, 2)));
+// Lets `kern` use `bytes` of dynamic shared memory, more than the 48 KB default (bytes < 0: the most
+// the device allows).  Set once per kernel and device; later calls return at once.
+int opt_in_dynamic_smem(const void* kern, int bytes);
 // Validates the problem description shared by the pair-batch entry points; `pitch_limit` = false skips
 // the pitch limits of the fused kernels (entry points that stage no shared-memory tile).
 int check_problem(const b200icp_problem* pr, int64_t n_pairs, bool pitch_limit = true);

@@ -1,5 +1,6 @@
 // compact.cuh -- order-preserving compaction (count -> exclusive scan -> scatter) of the points
-// i < n that a predicate keeps, shared by b200icp_select_points and b200icp_occ_filter_points.
+// i < n that a predicate keeps, shared by the point selection, the occupancy filter, the voxel grid
+// and the loop-closure entry points.
 #pragma once
 
 #include "common.cuh"
@@ -7,6 +8,9 @@
 namespace {   // kernels: instantiated in every translation unit that compacts
 
 constexpr int kCompactBlock = 1024;      // points per CTA (256 threads x 4)
+
+// length of compact()'s int64 scratch for n points: one count per CTA, then the total
+constexpr int64_t compact_scratch_len(int64_t n) { return (n + kCompactBlock - 1) / kCompactBlock + 1; }
 
 template <typename Keep>
 __global__ void __launch_bounds__(256) compact_count_kernel(const Keep keep, int64_t n, int64_t* block_counts) {
@@ -88,7 +92,7 @@ __global__ void __launch_bounds__(256) compact_scatter_kernel(const Keep keep, i
 }
 
 // emit(dst, i) for the dst-th of the points i < n with keep(i), in order; the count goes to
-// *count_out.  scratch: int64[ceil(n / 1024) + 1].  Launch errors name the kernels "<name>_count_kernel",
+// *count_out.  scratch: int64[compact_scratch_len(n)].  Launch errors name the kernels "<name>_count_kernel",
 // "<name>_scan_kernel" and "<name>_scatter_kernel".
 template <typename Keep, typename Emit>
 int compact(const Keep& keep, const Emit& emit, int64_t n, int64_t* scratch, int64_t* count_out,

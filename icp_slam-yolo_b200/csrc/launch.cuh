@@ -2,10 +2,6 @@
 // called by the dispatch of b200icp_nn_batch / b200icp_align_batch in b200icp.cu.
 #pragma once
 
-#include <mutex>
-#include <set>
-#include <utility>
-
 #include "common.cuh"
 
 struct LaunchShape {
@@ -28,27 +24,12 @@ int launch_pair_kernel(const b200icp_problem* prob, const LaunchShape& ls, Kerne
 int launch_nn_warp_kernel(const b200icp_problem* prob, const LaunchShape& ls, KernelArgs& args, bool dense,
                           cudaStream_t st);
 
-// One launch per call.  The opt-in to more than 48 KB of dynamic shared memory is made once per
-// kernel and device (the largest size the device allows), not on every launch.
+// One launch per call, opted in to the most dynamic shared memory the device allows when the shape
+// needs more than 48 KB.
 template <typename Kern, typename Args>
 int launch_pairs(Kern kern, const LaunchShape& ls, const Args& args, cudaStream_t st) {
-  if (ls.smem > 48 * 1024) {
-    // (all kernels share the function-pointer type, so the memo is keyed by pointer and device)
-    static std::mutex mu;
-    static std::set<std::pair<const void*, int>> opted_in;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::lock_guard<std::mutex> lock(mu);
-    const std::pair<const void*, int> key(reinterpret_cast<const void*>(kern), dev);
-    if (!opted_in.count(key)) {
-      int max_optin = 0;
-      cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin);
-      if (e != cudaSuccess)
-        return set_error(B200ICP_ERR_CUDA, "cudaFuncSetAttribute(max dynamic smem): %s", cudaGetErrorString(e));
-      opted_in.insert(key);
-    }
-  }
+  if (ls.smem > 48 * 1024)
+    if (const int rc = opt_in_dynamic_smem(reinterpret_cast<const void*>(kern), -1)) return rc;
   kern<<<(unsigned)args.n_pairs, ls.warps * 32, ls.smem, st>>>(args);
   return check_launch("kernel launch");
 }

@@ -2,7 +2,6 @@
 // information matrix of an alignment, graph edges from verified alignments and a batched float64
 // Gauss-Newton SE(2) pose-graph optimiser whose PCG solve runs on the device (DESIGN.md §4.9).
 // The reference has no loop closure: oracle/pose_graph_oracle.py defines the results.
-#include <cub/device/device_radix_sort.cuh>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -12,6 +11,7 @@
 #include <vector>
 
 #include "compact.cuh"
+#include "workspace.cuh"
 
 namespace {
 
@@ -485,31 +485,31 @@ __global__ void __launch_bounds__(kPgThreads) pose_graph_kernel(const PgArgs a) 
   }
 }
 
-// workspace layout (bytes, each part 256-aligned)
-struct PgLayout {
-  size_t offs, keys, vals, skeys, svals, rows, bad, edge_ws, node_ws, cub, total;
+struct PgBuffers {
+  void* ranges;             // node_offset[G + 1], edge_offset[G + 1] (int64), fixed[G] (int32): one copy
+  int32_t *keys, *vals;     // [2 * edges] node and edge of every edge slot
+  int32_t *skeys, *svals;   // the same, sorted by node
+  int32_t *rows, *bad;      // [nodes + 1], [G]
+  double *edge_ws, *node_ws;
+  SortTemp sort;
+  int64_t bytes;
 };
 
-size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
-PgLayout pg_layout(int64_t n_graphs, int64_t nodes, int64_t edges) {
-  PgLayout L;
-  size_t cub_bytes = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const int32_t*)nullptr, (int32_t*)nullptr,
-                                  (const int32_t*)nullptr, (int32_t*)nullptr, (int)(2 * edges));
-  size_t o = 0;
-  L.offs = o; o += align256(sizeof(int64_t) * (2 * (n_graphs + 1)) + sizeof(int32_t) * n_graphs);
-  L.keys = o; o += align256(sizeof(int32_t) * 2 * edges);
-  L.vals = o; o += align256(sizeof(int32_t) * 2 * edges);
-  L.skeys = o; o += align256(sizeof(int32_t) * 2 * edges);
-  L.svals = o; o += align256(sizeof(int32_t) * 2 * edges);
-  L.rows = o; o += align256(sizeof(int32_t) * (nodes + 1));
-  L.bad = o; o += align256(sizeof(int32_t) * n_graphs);
-  L.edge_ws = o; o += align256(sizeof(double) * kSlot * edges);
-  L.node_ws = o; o += align256(sizeof(double) * kNodeDoubles * nodes);
-  L.cub = o; o += align256(cub_bytes);
-  L.total = o;
-  return L;
+PgBuffers pg_buffers(void* base, int64_t n_graphs, int64_t nodes, int64_t edges) {
+  Carver c(base);
+  PgBuffers b;
+  b.ranges = c.take_bytes(sizeof(int64_t) * 2 * (n_graphs + 1) + sizeof(int32_t) * n_graphs);
+  b.keys = c.take<int32_t>(2 * edges);
+  b.vals = c.take<int32_t>(2 * edges);
+  b.skeys = c.take<int32_t>(2 * edges);
+  b.svals = c.take<int32_t>(2 * edges);
+  b.rows = c.take<int32_t>(nodes + 1);
+  b.bad = c.take<int32_t>(n_graphs);
+  b.edge_ws = c.take<double>(kSlot * edges);
+  b.node_ws = c.take<double>(kNodeDoubles * nodes);
+  b.sort = take_sort_temp<int32_t, int32_t>(c, 2 * edges);
+  b.bytes = c.total;
+  return b;
 }
 
 int pg_sizes(const b200icp_pose_graph_batch* g, int64_t& nodes, int64_t& edges) {
@@ -601,7 +601,7 @@ int b200icp_odometry_edges(int64_t n_pairs, const double* pose_total, const doub
 int64_t b200icp_pose_graph_workspace_bytes(const b200icp_pose_graph_batch* graphs) {
   int64_t nodes = 0, edges = 0;
   if (pg_sizes(graphs, nodes, edges) != B200ICP_OK) return -1;
-  return (int64_t)pg_layout(graphs->n_graphs, nodes, edges).total;
+  return pg_buffers(nullptr, graphs->n_graphs, nodes, edges).bytes;
 }
 
 int b200icp_pose_graph_optimize(const b200icp_pose_graph_batch* graphs, const b200icp_pose_graph_options* opt,
@@ -619,42 +619,35 @@ int b200icp_pose_graph_optimize(const b200icp_pose_graph_batch* graphs, const b2
   if (edges > 0 && (!graphs->edge_i || !graphs->edge_j || !graphs->meas || !graphs->info))
     return set_error(B200ICP_ERR_INVALID_ARGUMENT, "pose_graph: edge arrays are NULL");
   if (graphs->n_graphs == 0) return B200ICP_OK;
-  const PgLayout L = pg_layout(graphs->n_graphs, nodes, edges);
-  if (!workspace || workspace_bytes < (int64_t)L.total)
+  const int64_t G = graphs->n_graphs;
+  const PgBuffers b = pg_buffers(workspace, G, nodes, edges);
+  if (!workspace || workspace_bytes < b.bytes)
     return set_error(B200ICP_ERR_INVALID_ARGUMENT, "pose_graph: workspace smaller than b200icp_pose_graph_workspace_bytes()");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int64_t G = graphs->n_graphs;
-  char* ws = static_cast<char*>(workspace);
   // the ranges and the gauge nodes travel to the device once per call
   std::vector<char> host(sizeof(int64_t) * 2 * (G + 1) + sizeof(int32_t) * G);
   memcpy(host.data(), graphs->node_offset, sizeof(int64_t) * (G + 1));
   memcpy(host.data() + sizeof(int64_t) * (G + 1), graphs->edge_offset, sizeof(int64_t) * (G + 1));
   int32_t* hf = reinterpret_cast<int32_t*>(host.data() + sizeof(int64_t) * 2 * (G + 1));
   for (int64_t k = 0; k < G; ++k) hf[k] = graphs->fixed_node ? graphs->fixed_node[k] : 0;
-  cudaError_t e = cudaMemcpyAsync(ws + L.offs, host.data(), host.size(), cudaMemcpyHostToDevice, st);
+  cudaError_t e = cudaMemcpyAsync(b.ranges, host.data(), host.size(), cudaMemcpyHostToDevice, st);
   // (a copy from pageable memory is staged before cudaMemcpyAsync returns, so `host` may go out of scope)
   if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "pose_graph: ranges to the device: %s", cudaGetErrorString(e));
   PgGraphs pg;
-  pg.node_offset = reinterpret_cast<const int64_t*>(ws + L.offs);
+  pg.node_offset = static_cast<const int64_t*>(b.ranges);
   pg.edge_offset = pg.node_offset + (G + 1);
   pg.fixed = reinterpret_cast<const int32_t*>(pg.edge_offset + (G + 1));
-  int32_t* keys = reinterpret_cast<int32_t*>(ws + L.keys);
-  int32_t* vals = reinterpret_cast<int32_t*>(ws + L.vals);
-  int32_t* skeys = reinterpret_cast<int32_t*>(ws + L.skeys);
-  int32_t* svals = reinterpret_cast<int32_t*>(ws + L.svals);
-  int32_t* rows = reinterpret_cast<int32_t*>(ws + L.rows);
-  int32_t* bad = reinterpret_cast<int32_t*>(ws + L.bad);
   // ---- set-up: block-CSR of H (each node's slots in ascending edge order: the sort is stable)
-  pg_keys_kernel<<<(unsigned)G, 256, 0, st>>>(pg, graphs->edge_i, graphs->edge_j, nodes, keys, vals, bad);
+  pg_keys_kernel<<<(unsigned)G, 256, 0, st>>>(pg, graphs->edge_i, graphs->edge_j, nodes, b.keys, b.vals, b.bad);
   if (const int rc = check_launch("pg_keys_kernel")) return rc;
   if (edges > 0) {
-    size_t cub_bytes = L.total - L.cub;
     int bits = 1;
     while (bits < 31 && (1LL << bits) <= nodes) ++bits;
-    e = cub::DeviceRadixSort::SortPairs(ws + L.cub, cub_bytes, keys, skeys, vals, svals, (int)(2 * edges), 0, bits, st);
-    if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "pose_graph: radix sort: %s", cudaGetErrorString(e));
+    if (const int rc = radix_sort_pairs(b.sort, b.keys, b.skeys, b.vals, b.svals, 2 * edges, 0, bits, st,
+                                        "pose_graph: radix sort"))
+      return rc;
   }
-  pg_rows_kernel<<<(unsigned)((nodes + 256) / 256), 256, 0, st>>>(skeys, 2 * edges, nodes, rows);
+  pg_rows_kernel<<<(unsigned)((nodes + 256) / 256), 256, 0, st>>>(b.skeys, 2 * edges, nodes, b.rows);
   if (const int rc = check_launch("pg_rows_kernel")) return rc;
   if (nodes > 0) {
     e = cudaMemcpyAsync(out->poses, graphs->poses_in, sizeof(double) * 6 * nodes, cudaMemcpyDeviceToDevice, st);
@@ -666,11 +659,11 @@ int b200icp_pose_graph_optimize(const b200icp_pose_graph_batch* graphs, const b2
   args.ej = graphs->edge_j;
   args.meas = graphs->meas;
   args.info = graphs->info;
-  args.row_ptr = rows;
-  args.slot_edge = svals;
-  args.bad = bad;
-  args.edge_ws = reinterpret_cast<double*>(ws + L.edge_ws);
-  args.node_ws = reinterpret_cast<double*>(ws + L.node_ws);
+  args.row_ptr = b.rows;
+  args.slot_edge = b.svals;
+  args.bad = b.bad;
+  args.edge_ws = b.edge_ws;
+  args.node_ws = b.node_ws;
   args.opt = *opt;
   args.out = *out;
   pose_graph_kernel<<<(unsigned)G, kPgThreads, 0, st>>>(args);

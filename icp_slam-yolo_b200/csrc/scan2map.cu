@@ -40,14 +40,13 @@
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
-#include <cub/cub.cuh>
-
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
 
 #include "common.cuh"
+#include "workspace.cuh"
 
 namespace {
 
@@ -167,26 +166,24 @@ __global__ void __launch_bounds__(256) s2m_gather_kernel(const void* points, int
   else reinterpret_cast<float2*>(sorted)[j] = reinterpret_cast<const float2*>(points)[order[j]];
 }
 
-struct SortWs {
-  int64_t box, keys_in, keys_out, idx_in, cub, total;
-  size_t cub_bytes;
+struct MortonBuffers {
+  unsigned long long* box;
+  unsigned *keys_in, *keys_out;
+  int32_t* idx_in;
+  SortTemp sort;
+  int64_t bytes;
 };
 
-SortWs sort_layout(int64_t m) {
-  auto up = [](int64_t b) { return (b + 255) / 256 * 256; };
-  SortWs w;
-  size_t cub_bytes = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned*)nullptr, (unsigned*)nullptr,
-                                  (const int32_t*)nullptr, (int32_t*)nullptr, (int)m);
-  w.cub_bytes = cub_bytes;
-  int64_t off = 0;
-  w.box = off;      off += 256;
-  w.keys_in = off;  off += up(m * 4);
-  w.keys_out = off; off += up(m * 4);
-  w.idx_in = off;   off += up(m * 4);
-  w.cub = off;      off += up((int64_t)cub_bytes);
-  w.total = off;
-  return w;
+MortonBuffers morton_buffers(void* base, int64_t m) {
+  Carver c(base);
+  MortonBuffers b;
+  b.box = c.take<unsigned long long>(4);
+  b.keys_in = c.take<unsigned>(m);
+  b.keys_out = c.take<unsigned>(m);
+  b.idx_in = c.take<int32_t>(m);
+  b.sort = take_sort_temp<unsigned, int32_t>(c, m);
+  b.bytes = c.total;
+  return b;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -900,7 +897,7 @@ int64_t b200icp_s2m_inbox_bytes(int32_t n_scan, int32_t world) {
 
 int64_t b200icp_s2m_prepare_workspace_bytes(int64_t m) {
   if (m < 1 || m > 0x7fffffffLL) return -1;
-  return sort_layout(m).total;
+  return morton_buffers(nullptr, m).bytes;
 }
 
 int b200icp_s2m_prepare_map(const b200icp_s2m_shard* shard, void* workspace, int64_t workspace_bytes,
@@ -919,22 +916,16 @@ int b200icp_s2m_prepare_map(const b200icp_s2m_shard* shard, void* workspace, int
   const void* scanned = shard->points;
   if (shard->sorted_points) {                   // Morton order (see above)
     if (shard->m > 0x7fffffffLL) return set_error(B200ICP_ERR_UNSUPPORTED_SHAPE, "s2m_prepare_map: spatial sort needs m < 2^31");
-    const SortWs w = sort_layout(shard->m);
-    if (!workspace || workspace_bytes < w.total) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: workspace too small");
-    unsigned char* base = reinterpret_cast<unsigned char*>(workspace);
-    unsigned long long* box = reinterpret_cast<unsigned long long*>(base + w.box);
-    unsigned* keys_in = reinterpret_cast<unsigned*>(base + w.keys_in);
-    unsigned* keys_out = reinterpret_cast<unsigned*>(base + w.keys_out);
-    int32_t* idx_in = reinterpret_cast<int32_t*>(base + w.idx_in);
-    if (cudaMemsetAsync(box, 0xff, 16, st) != cudaSuccess || cudaMemsetAsync(box + 2, 0, 16, st) != cudaSuccess)
+    const MortonBuffers b = morton_buffers(workspace, shard->m);
+    if (!workspace || workspace_bytes < b.bytes) return set_error(B200ICP_ERR_INVALID_ARGUMENT, "s2m_prepare_map: workspace too small");
+    if (cudaMemsetAsync(b.box, 0xff, 16, st) != cudaSuccess || cudaMemsetAsync(b.box + 2, 0, 16, st) != cudaSuccess)
       return check_launch("cudaMemsetAsync");
     const unsigned blocks = (unsigned)((shard->m + 255) / 256);
-    s2m_bbox_kernel<<<blocks < 1184u ? blocks : 1184u, 256, 0, st>>>(shard->points, shard->dtype, shard->m, box);
-    s2m_morton_kernel<<<blocks, 256, 0, st>>>(shard->points, shard->dtype, shard->m, box, keys_in, idx_in);
-    size_t cub_bytes = w.cub_bytes;
-    cudaError_t e = cub::DeviceRadixSort::SortPairs(base + w.cub, cub_bytes, keys_in, keys_out, idx_in, shard->order,
-                                                    (int)shard->m, 0, 32, st);
-    if (e != cudaSuccess) return set_error(B200ICP_ERR_CUDA, "%s", cudaGetErrorString(e));
+    s2m_bbox_kernel<<<blocks < 1184u ? blocks : 1184u, 256, 0, st>>>(shard->points, shard->dtype, shard->m, b.box);
+    s2m_morton_kernel<<<blocks, 256, 0, st>>>(shard->points, shard->dtype, shard->m, b.box, b.keys_in, b.idx_in);
+    if (const int rc = radix_sort_pairs(b.sort, b.keys_in, b.keys_out, b.idx_in, shard->order, shard->m, 0, 32, st,
+                                        "s2m_prepare_map: radix sort"))
+      return rc;
     s2m_gather_kernel<<<blocks, 256, 0, st>>>(shard->points, shard->dtype, shard->m, shard->order, shard->sorted_points);
     int rc = check_launch("s2m spatial sort");
     if (rc) return rc;

@@ -3,13 +3,12 @@ loop, on the device: the local-map radius crop (duc/ICP_LIDAR/mainn.py:297-308) 
 removal (duc/ICP_LIDAR/process.py:75-84).  Both keep the input order."""
 from __future__ import annotations
 
-import ctypes as C
 from typing import Optional
 
 import torch
 
 from . import _cabi
-from .registration import _DTYPES, ScanTable, _ptr, _require_cuda, _stream_ptr, nn_search
+from .registration import _DTYPES, ScanTable, _compact_scratch, _ptr, _require_cuda, _stream_ptr, _workspace, nn_search
 
 
 def _select(points: torch.Tensor, mode: int, key: Optional[torch.Tensor], cx: float, cy: float,
@@ -20,11 +19,10 @@ def _select(points: torch.Tensor, mode: int, key: Optional[torch.Tensor], cx: fl
     n = int(points.shape[0])
     out = torch.empty_like(points)
     count = torch.zeros(1, dtype=torch.int64, device=points.device)
-    scratch = torch.empty((n + 1023) // 1024 + 1, dtype=torch.int64, device=points.device)
     with torch.cuda.device(points.device):
         rc = _cabi.lib().b200icp_select_points(_ptr(points), _DTYPES[points.dtype], n, mode, _ptr(key),
                                                float(cx), float(cy), float(threshold), _ptr(out),
-                                               _ptr(count), _ptr(scratch), _stream_ptr(stream))
+                                               _ptr(count), _ptr(_compact_scratch(n, points.device)), _stream_ptr(stream))
     _cabi.check(rc, "b200icp_select_points")
     return out[: int(count.item())]
 
@@ -70,13 +68,11 @@ def voxel_down_sample(points: torch.Tensor, voxel_size: float, stream=None) -> t
     n = int(points.shape[0])
     if n == 0:
         return points
-    lib = _cabi.lib()
-    wb = lib.b200icp_voxel_workspace_bytes(n)
-    ws = torch.empty(wb, dtype=torch.uint8, device=points.device)
+    ws, wb = _workspace(_cabi.lib().b200icp_voxel_workspace_bytes, n, device=points.device)
     out = torch.empty_like(points)
     count = torch.zeros(1, dtype=torch.int64, device=points.device)
     with torch.cuda.device(points.device):
-        rc = lib.b200icp_voxel_downsample(_ptr(points), _DTYPES[points.dtype], n, float(voxel_size), _ptr(out),
-                                          _ptr(count), _ptr(ws), wb, _stream_ptr(stream))
+        rc = _cabi.lib().b200icp_voxel_downsample(_ptr(points), _DTYPES[points.dtype], n, float(voxel_size),
+                                                  _ptr(out), _ptr(count), _ptr(ws), wb, _stream_ptr(stream))
     _cabi.check(rc, "b200icp_voxel_downsample")
     return out[: int(count.item())]

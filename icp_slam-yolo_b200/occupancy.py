@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .registration import _DTYPES, _ptr, _require_cuda, _stream_ptr
+from .registration import _DTYPES, _compact_scratch, _ptr, _require_cuda, _stream_ptr
 
 THRESHOLD_UP = 0.65              # process.py:158
 
@@ -124,12 +124,11 @@ class OccupancyGrid:
         n, cols = int(pts.shape[0]), int(pts.shape[1])
         kept = torch.empty(n, dtype=torch.int64, device=dev)
         count = torch.zeros(1, dtype=torch.int64, device=dev)
-        scratch = torch.empty((n + 1023) // 1024 + 1, dtype=torch.int64, device=dev)
         with torch.cuda.device(dev):
             rc = _cabi.lib().b200icp_occ_filter_points(
                 _ptr(pts), _DTYPES[pts.dtype], cols, n, _ptr(self.probs[map_index]), self.h, self.w,
                 self.center[0], self.center[1], self.resolution, _f32(free_threshold), _ptr(kept),
-                _ptr(count), _ptr(scratch), _stream_ptr(stream))
+                _ptr(count), _ptr(_compact_scratch(n, dev)), _stream_ptr(stream))
         _cabi.check(rc, "b200icp_occ_filter_points")
         idx = kept[: int(count.item())]
         return points[idx.cpu().numpy()] if as_numpy else points[idx]

@@ -17,18 +17,14 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .registration import AlignResult, ScanTable, _check_pairs, _default_pairs, _problem, _ptr, _require_cuda, \
-    _stream_ptr, align_pairs
+from .registration import AlignResult, ScanTable, _check_pairs, _compact_scratch, _default_pairs, _problem, _ptr, \
+    _require_cuda, _stream_ptr, _workspace, align_pairs
 
 
 def _pose_table(t: torch.Tensor, name: str) -> None:
     if t.dtype != torch.float64 or t.dim() != 2 or t.shape[1] != 6:
         raise ValueError(f"{name} must be float64 [n, 6], got {t.dtype} {tuple(t.shape)}")
     _require_cuda(t, name)
-
-
-def _scratch(n: int, dev) -> torch.Tensor:
-    return torch.empty((n + 1023) // 1024 + 1, dtype=torch.int64, device=dev)
 
 
 def loop_candidates(poses: torch.Tensor, min_gap: int, radius: float, *, capacity: Optional[int] = None,
@@ -43,7 +39,7 @@ def loop_candidates(poses: torch.Tensor, min_gap: int, radius: float, *, capacit
     if cap < 0:
         raise ValueError("capacity < 0")
     count = torch.empty(1, dtype=torch.int64, device=dev)
-    scratch = _scratch(n * (n - 1) // 2, dev)
+    scratch = _compact_scratch(n * (n - 1) // 2, dev)
     while True:
         src = torch.empty(cap, dtype=torch.int32, device=dev)
         tgt = torch.empty(cap, dtype=torch.int32, device=dev)
@@ -160,7 +156,7 @@ class PoseGraph:
         with torch.cuda.device(dev):
             rc = _cabi.lib().b200icp_odometry_edges(b, _ptr(result.pose_total), _ptr(result.error),
                                                     _ptr(result.iterations), _info_ptr(info, b), _ptr(ei), _ptr(ej),
-                                                    _ptr(meas), _ptr(inf), _ptr(count), _ptr(_scratch(b, dev)),
+                                                    _ptr(meas), _ptr(inf), _ptr(count), _ptr(_compact_scratch(b, dev)),
                                                     _stream_ptr(stream))
         _cabi.check(rc, "b200icp_odometry_edges")
         k = int(count.item())
@@ -188,7 +184,7 @@ class PoseGraph:
             rc = _cabi.lib().b200icp_loop_edges(b, _ptr(result.pose_total), _ptr(result.rmse), _ptr(result.inliers),
                                                 _ptr(src_lengths), pitch, _ptr(src_row), _ptr(tgt_row),
                                                 _info_ptr(info, b), float(min_fitness), float(max_rmse), _ptr(ei),
-                                                _ptr(ej), _ptr(meas), _ptr(inf), _ptr(count), _ptr(_scratch(b, dev)),
+                                                _ptr(ej), _ptr(meas), _ptr(inf), _ptr(count), _ptr(_compact_scratch(b, dev)),
                                                 _stream_ptr(stream))
         _cabi.check(rc, "b200icp_loop_edges")
         k = int(count.item())
@@ -284,13 +280,14 @@ def optimize_pose_graph(graphs: Union[PoseGraph, Sequence[PoseGraph]],
     out.iterations, out.pcg_iterations = res.iterations.data_ptr(), res.pcg_iterations.data_ptr()
     out.status, out.isolated, out.anchored = res.status.data_ptr(), res.isolated.data_ptr(), res.anchored.data_ptr()
     L = _cabi.lib()
-    nbytes = L.b200icp_pose_graph_workspace_bytes(C.byref(batch))
-    if nbytes < 0:
-        _cabi.check(_cabi.lib().b200icp_pose_graph_optimize(C.byref(batch), C.byref(opt), C.byref(out), None, 0, None),
+    try:
+        ws, nbytes = _workspace(L.b200icp_pose_graph_workspace_bytes, C.byref(batch), device=dev)
+    except _cabi.B200IcpError:              # the optimiser's own checks say what is wrong with the batch
+        _cabi.check(L.b200icp_pose_graph_optimize(C.byref(batch), C.byref(opt), C.byref(out), None, 0, None),
                     "b200icp_pose_graph_optimize")
-    ws = torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=dev)
+        raise
     with torch.cuda.device(dev):
-        rc = L.b200icp_pose_graph_optimize(C.byref(batch), C.byref(opt), C.byref(out), _ptr(ws), int(nbytes),
+        rc = L.b200icp_pose_graph_optimize(C.byref(batch), C.byref(opt), C.byref(out), _ptr(ws), nbytes,
                                            _stream_ptr(stream))
     _cabi.check(rc, "b200icp_pose_graph_optimize")
     return res

@@ -131,6 +131,17 @@ def _stream_ptr(stream) -> C.c_void_p:
     return C.c_void_p(s.cuda_stream)
 
 
+def _compact_scratch(n: int, device) -> torch.Tensor:
+    return torch.empty((n + 1023) // 1024 + 1, dtype=torch.int64, device=device)   # compact.cuh: a count per 1,024
+
+
+def _workspace(query, *args, device):        # query: a b200icp_*_workspace_bytes function
+    nbytes = int(query(*args))
+    if nbytes < 0:
+        raise _cabi.B200IcpError(f"{query.__name__} failed")
+    return torch.empty(max(nbytes, 1), dtype=torch.uint8, device=device), nbytes
+
+
 def _problem(src: ScanTable, tgt: ScanTable, pairing: str, src_row, tgt_row, first_pair: int):
     if src.points.dtype != tgt.points.dtype:
         raise ValueError("source and target tables must share a dtype")

@@ -22,7 +22,7 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .registration import _DTYPES, _ptr, _require_cuda, _stream_ptr
+from .registration import _DTYPES, _ptr, _require_cuda, _stream_ptr, _workspace
 
 RECORD_BYTES = 32
 STATE_BYTES = 136
@@ -75,12 +75,8 @@ class MapShard:
             self._prepare(stream)
 
     def _prepare(self, stream):
-        ws, nbytes = None, 0
-        if self.order is not None:
-            nbytes = int(_lib().b200icp_s2m_prepare_workspace_bytes(self.m))
-            if nbytes < 0:
-                raise _cabi.B200IcpError("b200icp_s2m_prepare_workspace_bytes failed")
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=self.points.device)
+        ws, nbytes = (None, 0) if self.order is None else \
+            _workspace(_lib().b200icp_s2m_prepare_workspace_bytes, self.m, device=self.points.device)
         with torch.cuda.device(self.points.device):
             rc = _lib().b200icp_s2m_prepare_map(C.byref(self.desc), _ptr(ws), nbytes, _stream_ptr(stream))
         _cabi.check(rc, "b200icp_s2m_prepare_map")
